@@ -4,6 +4,7 @@ configuration: Book-2 final scene, 800x800, 10,000 spp, max_depth 40 (config C5)
 
     python bench.py --gpus N --steps K --warmup W            # our arm (torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path, host cores
+    python bench.py ... --dump-outputs DIR                   # + the image of the last timed step, DIR/radiance.npy
 
 One STEP = one full render of the workload: every rank renders its shard of the sample indices
 of every pixel (strong scaling: the job is fixed, N ranks split the 10,000 spp), then the exact
@@ -88,7 +89,32 @@ def parse():
     ap.add_argument("--reduce", default="peer", choices=["peer", "nccl"],
                     help="N > 1: 'peer' = behind its render kernel every rank adds its accumulator into rank 0's buffer with our own "
                          "push kernel (peer memory over NVLink, CUDA IPC, no collective); 'nccl' = ncclInt64 reduce")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the image the last one rendered (rank 0's reduced radiance, float32 H x W x 3) "
+                         "to DIR/radiance.npy; above 64 MB, a fixed seeded sample of its pixels, their flat indices in DIR/pixel_index.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
+
+
+DUMP_LIMIT = 64 << 20  # bytes of .npy files --dump-outputs may write
+
+
+def dump_outputs(out_dir, radiance):
+    """radiance.npy = the H x W x 3 image, or, when that exceeds DUMP_LIMIT, the pixels at a fixed seeded sample of flat
+    indices (pixel_index.npy, ascending) — the same files for the same arguments, so two builds compare output for output."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    if radiance.nbytes > DUMP_LIMIT:
+        n = (DUMP_LIMIT - 4096) // (3 * radiance.itemsize + 8)
+        idx = np.sort(np.random.default_rng(0).choice(radiance.shape[0] * radiance.shape[1], n, replace=False))
+        np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+        radiance = radiance.reshape(-1, 3)[idx]
+    np.save(os.path.join(out_dir, "radiance.npy"), radiance)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -375,6 +401,8 @@ def main():
     wall = time.time() - t_wall0
     clocks = sampler.summary()
     launches = ctx.stats().kernel_launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx.download_radiance(spp))
 
     # ---- e2e: the reference-facing C-ABI call sequence with host buffers ---------------------
     e2e_steps = args.steps

@@ -1,3 +1,4 @@
+import hashlib
 import importlib
 import json
 import os
@@ -8,6 +9,26 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+
+# The scenes with an image texture ("earth", "book2_final") load earthmap.jpg from RTW_IMAGES.  The reference's image is
+# not part of this repository.  When RTW_IMAGES holds it (recognised by its sha256 in ref_pins.json), the tests compare
+# with the reference's own pins; otherwise they read a generated stand-in of the same size and format
+# (tests/golden/make_standin.py) and compare with the pins taken on it.  EARTHMAP holds whichever pins apply.
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+
+
+def _earthmap_pins():
+    ref = json.load(open(os.path.join(GOLDEN, "ref_pins.json")))
+    d = os.environ.get("RTW_IMAGES", "")
+    path = os.path.join(d, "earthmap.jpg")
+    if d and os.path.isfile(path) and hashlib.sha256(open(path, "rb").read()).hexdigest() == ref["earthmap"]["jpeg_sha256"]:
+        return dict(ref["earthmap"], dir=d, small={n: s["ppm"]["sha256"] for n, s in ref["scenes"].items()},
+                    shipped={n: s["ppm_sha256"] for n, s in ref["shipped"].items()})
+    return dict(json.load(open(os.path.join(GOLDEN, "earthmap_standin.json"))), dir=os.path.join(GOLDEN, "images"))
+
+
+EARTHMAP = _earthmap_pins()
+os.environ["RTW_IMAGES"] = EARTHMAP["dir"]
 
 
 def pytest_configure(config):
@@ -37,6 +58,12 @@ def orc():
 def pins():
     with open(os.path.join(ROOT, "tests", "golden", "ref_pins.json")) as f:
         return json.load(f)
+
+
+@pytest.fixture(scope="session")
+def earthmap():
+    """Pins of the earthmap.jpg the tests render with: the reference's image when RTW_IMAGES holds it, else the stand-in."""
+    return EARTHMAP
 
 
 @pytest.fixture(scope="session")

@@ -77,13 +77,11 @@ def test_perlin_marble(rtb, orc, gpu_ctx):
         assert err.mean() <= 5e-5
 
 
-def test_earth_texture_through_named_scene(rtb, orc, gpu_ctx, pins):
-    """The real earthmap.jpg through the host JPEG decoder + rtw_image conventions."""
-    if rtb.default_image_dir() is None:
-        pytest.skip("earthmap.jpg is not available on this machine")
+def test_earth_texture_through_named_scene(rtb, orc, gpu_ctx, earthmap):
+    """The earth scene's earthmap.jpg (the reference's or the stand-in, conftest.py) through the host JPEG decoder + rtw_image conventions."""
     sc = rtb.Scene("earth", rand_seed=1)
     d = sc.desc.contents
-    assert d.n_images == 1 and d.images[0].width == pins["earthmap"]["width"] and d.images[0].height == pins["earthmap"]["height"]
+    assert d.n_images == 1 and d.images[0].width == earthmap["width"] and d.images[0].height == earthmap["height"]
     gpu_ctx.upload_scene(sc.desc)
     rng = np.random.default_rng(4)
     uvp = _points(rng, 100_000, 1.0)
