@@ -319,12 +319,42 @@ int rt_trace_rays(rt_ctx* ctx, int64_t n, const double* origin, const double* di
                   const double* time, double tmin, double tmax, int32_t flags,
                   int32_t* prim_id, double* t, double* normal, uint8_t* front_face);
 
+/* rt_trace_rays for rays that start ON a primitive, as every ray after the first of a path
+ * does in rt_render: start_prim[i] is the reference primitive id (rt_hittable.prim_id) ray i
+ * leaves from, or -1 for none, and the traversal applies rt_render's start-primitive rules
+ * instead of an epsilon (a sphere gets the roots 0 and -2b/a, a quad is skipped, a box face's
+ * slab plane is crossed at exactly 0).  start_prim == NULL is rt_trace_rays.  FP32 mode
+ * only: RT_TRACE_EXACT with a start_prim is RT_ERR_INVALID (the reference has no start
+ * primitive), and so is an id that is not a primitive of the device BVH (the boundary of a
+ * medium, say) or that names more than one device primitive.                           */
+int rt_trace_rays_from(rt_ctx* ctx, int64_t n, const double* origin, const double* direction,
+                       const double* time, const int32_t* start_prim, double tmin, double tmax,
+                       int32_t flags, int32_t* prim_id, double* t, double* normal,
+                       uint8_t* front_face);
+
 /* Pixel-centre primary rays (no jitter, no defocus, time 0, interval (0.001, inf)),
  * generated on the device from the camera frame: SURVEY.md §8(c) convention.  With
  * RT_TRACE_RENDER_KERNEL the rays are the fp32 rays the render kernel builds (get_ray
  * at zero jitter) and t / normal are its fp32 results widened to double.               */
 int rt_primary_visibility(rt_ctx* ctx, const rt_camera_desc* cam, int32_t flags,
                           int32_t* prim_id, double* t, double* normal);
+
+/* The render kernel's first TWO segments of the pixel-centre path, traced by render_kernel
+ * itself (its AOV instantiation under the plan rt_render picks for the scene; media
+ * transparent, time 0).  Where the pixel-centre ray hits, the kernel shades the hit as
+ * rt_render does (surface_at + material scatter with the Philox stream of sample 0 of the
+ * pixel under `seed`, bounce 1), starts the scattered ray on that primitive (rt_render's
+ * start-primitive rule) and traces it with the same traversal.  Per pixel (row-major, any
+ * output may be NULL): prim_id / t of the primary hit (-1 / inf on a miss); origin1 /
+ * dir1 = the fp32 bounce ray (3 floats each, 0 without one); bounce_id / bounce_t /
+ * bounce_normal / bounce_front = its closest hit as in rt_trace_rays, bounce_id =
+ * RT_NO_BOUNCE when there is no bounce ray (primary miss, or the material absorbed or
+ * emitted: a light, a metal ray scattered below the surface).                          */
+enum { RT_NO_BOUNCE = -2147483647 - 1 };
+int rt_bounce_visibility(rt_ctx* ctx, const rt_camera_desc* cam, uint64_t seed,
+                         int32_t* prim_id, double* t, float* origin1, float* dir1,
+                         int32_t* bounce_id, double* bounce_t, double* bounce_normal,
+                         uint8_t* bounce_front);
 
 /* Entry/exit parameters (rec1.t, rec2.t of SURVEY.md App. B.2, before clamping) of the
  * boundary of the medium_index-th RT_H_MEDIUM (DFS order) for n rays; NaN when missed. */

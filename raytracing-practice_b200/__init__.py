@@ -63,7 +63,9 @@ def cuda_lib():
         lib.rt_camera_initialize.argtypes = [C.POINTER(_abi.rt_camera_desc), C.POINTER(_abi.rt_camera_frame)]
         dp, ip, bp, fp = C.POINTER(C.c_double), C.POINTER(C.c_int32), C.POINTER(C.c_uint8), C.POINTER(C.c_float)
         lib.rt_trace_rays.argtypes = [C.c_void_p, C.c_int64, dp, dp, dp, C.c_double, C.c_double, C.c_int32, ip, dp, dp, bp]
+        lib.rt_trace_rays_from.argtypes = [C.c_void_p, C.c_int64, dp, dp, dp, ip, C.c_double, C.c_double, C.c_int32, ip, dp, dp, bp]
         lib.rt_primary_visibility.argtypes = [C.c_void_p, C.POINTER(_abi.rt_camera_desc), C.c_int32, ip, dp, dp]
+        lib.rt_bounce_visibility.argtypes = [C.c_void_p, C.POINTER(_abi.rt_camera_desc), C.c_uint64, ip, dp, fp, fp, ip, dp, dp, bp]
         lib.rt_medium_spans.argtypes = [C.c_void_p, C.c_int32, C.c_int64, dp, dp, dp, dp, dp]
         lib.rt_eval_texture.argtypes = [C.c_void_p, C.c_int32, C.c_int64, dp, fp]
         lib.rt_eval_scatter.argtypes = [C.c_void_p, C.c_int32, C.c_int64, C.c_uint64, dp, dp, bp, fp, fp, bp]
@@ -239,7 +241,9 @@ class Context:
         s = self.stats()
         return self._download(RT_BUF_RGB8, spp, np.empty((s.image_height, s.image_width, 3), np.uint8))
 
-    def trace_rays(self, origin, direction, time=None, tmin=0.001, tmax=float("inf"), flags=RT_TRACE_FP32):
+    def trace_rays(self, origin, direction, time=None, tmin=0.001, tmax=float("inf"), flags=RT_TRACE_FP32, start_prim=None):
+        """start_prim: per ray the primitive id it starts on (-1: none), for rays that leave a surface as rt_render's
+        bounce rays do (rt_trace_rays_from; fp32 mode only)."""
         origin = np.ascontiguousarray(origin, np.float64)
         direction = np.ascontiguousarray(direction, np.float64)
         n = origin.shape[0]
@@ -248,10 +252,17 @@ class Context:
         t = np.empty(n, np.float64)
         nrm = np.empty((n, 3), np.float64)
         ff = np.empty(n, np.uint8)
-        rc = self._lib.rt_trace_rays(
-            self._h, n, _dptr(origin), _dptr(direction), _dptr(time), tmin, tmax, flags,
-            ids.ctypes.data_as(C.POINTER(C.c_int32)), _dptr(t), _dptr(nrm), ff.ctypes.data_as(C.POINTER(C.c_uint8)))
-        self._check(rc, "rt_trace_rays")
+        ip = C.POINTER(C.c_int32)
+        sp = None
+        if start_prim is not None:
+            start_prim = np.ascontiguousarray(start_prim, np.int32)
+            if start_prim.shape != (n,):
+                raise ValueError(f"start_prim must hold one id per ray: shape {start_prim.shape}, {n} rays")
+            sp = start_prim.ctypes.data_as(ip)
+        rc = self._lib.rt_trace_rays_from(
+            self._h, n, _dptr(origin), _dptr(direction), _dptr(time), sp, tmin, tmax, flags,
+            ids.ctypes.data_as(ip), _dptr(t), _dptr(nrm), ff.ctypes.data_as(C.POINTER(C.c_uint8)))
+        self._check(rc, "rt_trace_rays_from")
         return ids, t, nrm, ff
 
     def primary_visibility(self, cam, flags=RT_TRACE_EXACT | RT_TRACE_SKIP_MEDIA):
@@ -262,6 +273,19 @@ class Context:
         rc = self._lib.rt_primary_visibility(self._h, C.byref(cam), flags, ids.ctypes.data_as(C.POINTER(C.c_int32)), _dptr(t), _dptr(nrm))
         self._check(rc, "rt_primary_visibility")
         return ids, t, nrm
+
+    def bounce_visibility(self, cam, seed=0):
+        """The render kernel's first two segments of every pixel-centre path (rt_bounce_visibility), as a dict of H x W
+        arrays: id, t (primary hit); o1, d1 (fp32 bounce ray); id1, t1, n1, front1 (its hit; id1 = RT_NO_BOUNCE without one)."""
+        w, h = cam.image_width, image_height(cam)
+        out = dict(id=np.empty((h, w), np.int32), t=np.empty((h, w)), o1=np.empty((h, w, 3), np.float32), d1=np.empty((h, w, 3), np.float32),
+                   id1=np.empty((h, w), np.int32), t1=np.empty((h, w)), n1=np.empty((h, w, 3)), front1=np.empty((h, w), np.uint8))
+        ip, fp = C.POINTER(C.c_int32), C.POINTER(C.c_float)
+        rc = self._lib.rt_bounce_visibility(self._h, C.byref(cam), seed, out["id"].ctypes.data_as(ip), _dptr(out["t"]), out["o1"].ctypes.data_as(fp),
+                                            out["d1"].ctypes.data_as(fp), out["id1"].ctypes.data_as(ip), _dptr(out["t1"]), _dptr(out["n1"]),
+                                            out["front1"].ctypes.data_as(C.POINTER(C.c_uint8)))
+        self._check(rc, "rt_bounce_visibility")
+        return out
 
     def medium_spans(self, medium_index, origin, direction, time=None):
         origin = np.ascontiguousarray(origin, np.float64)

@@ -17,6 +17,7 @@ RT_T_SOLID, RT_T_CHECKER, RT_T_IMAGE, RT_T_NOISE = 1, 2, 3, 4
 
 RT_BUF_ACCUM_I64, RT_BUF_RADIANCE_F32, RT_BUF_RGB8 = 0, 1, 2
 RT_TRACE_FP32, RT_TRACE_EXACT, RT_TRACE_SKIP_MEDIA, RT_TRACE_RENDER_KERNEL = 0, 1, 2, 4
+RT_NO_BOUNCE = -(2 ** 31)  # rt_bounce_visibility: no bounce ray
 RT_RENDER_DEFAULT, RT_RENDER_COUNTERS, RT_RENDER_MEGAKERNEL, RT_RENDER_STREAM, RT_RENDER_REFILL = 0, 1, 2, 8, 16
 
 
@@ -178,7 +179,9 @@ C_ABI_SYMBOLS = [
     "rt_upload_accum",
     "rt_get_stats",
     "rt_trace_rays",
+    "rt_trace_rays_from",
     "rt_primary_visibility",
+    "rt_bounce_visibility",
     "rt_medium_spans",
     "rt_eval_texture",
     "rt_eval_scatter",

@@ -66,6 +66,7 @@ struct RenderParams {
   int* aov_id;             // render_kernel<.., AOV>: primitive id, t and shading normal of every pixel-centre ray
   float* aov_t;
   float* aov_n;
+  float* aov_b;            // render_kernel<.., AOV> with max_depth 2: the bounce segment, kAovBounce floats per pixel
   StreamLayout sl;   // streaming kernel only
 };
 
@@ -91,6 +92,7 @@ constexpr int RT_RENDER_POOL_REMOVED = 4;  // rt_b200.h: the bit of the removed 
 #endif
 constexpr bool kDefaultRefillKernel = RT_DEFAULT_REFILL != 0;
 constexpr float kFixScale = 4294967296.0f;  // 2^32
+constexpr int kAovBounce = 12;              // floats per pixel of the bounce AOV record (render_kernel)
 
 __device__ __forceinline__ long long to_fixed(float v) {
   // NaN -> 0 (a NaN sample would poison the pixel).  The clamp bounds one sample at 2^16 = 65,536 (the brightest
@@ -119,7 +121,10 @@ __global__ void push_kernel(const unsigned long long* __restrict__ accum, unsign
 // work distribution, camera ray arithmetic, closest_hit_keyfn with the same node / leaf steps and stack — traces the
 // jitter-free pixel-centre ray of every pixel (no defocus, time 0, media transparent) and, instead of shading, writes
 // the primitive id, t and normal it found, so that the traversal rt_render runs is itself under the id / t / normal gate
-// (camera.hpp:192, hittable_list.hpp:40-64).
+// (camera.hpp:192, hittable_list.hpp:40-64).  With P.aov_b (rt_bounce_visibility, max_depth 2) a pixel-centre ray that
+// hits is shaded as rt_render shades it (surface_at + scatter_ray, sample 0, bounce 1), its scattered ray takes the
+// start primitive exactly as below (`skip`) and goes through the same traversal in the next iteration; that second hit
+// is written as the record {origin1.xyz, dir1.xyz, normal.xyz, t, id bits, front}.
 // COOP = true evaluates Perlin turbulence warp-cooperatively (below); chosen per scene by the launch plan — only where a
 // good share of the primitives carries a noise texture: the hoisted hit record it needs costs the other scenes 3 %.
 template <bool COUNT, bool ALL_SMEM, bool SSTACK = false, bool AOV = false, bool COOP = false>
@@ -254,14 +259,17 @@ __global__ void __launch_bounds__(kRenderThreads, 1) render_kernel(const __grid_
       t = tt, sk = __float_as_uint(ss);
     };
     Hit h = closest_hit_keyfn<COUNT, ALL_SMEM>(sc, ns, o, d, 0.001f, INF, media, key_of, aux_of, cn, alive, ls, st);
-    if (AOV) {
+    if constexpr (AOV) {
       if (alive) {
-        const int pixel = __float_as_int(lds_f4(st_a + kStB).x);
+        const float4 A = lds_f4(st_a), B = lds_f4(st_a + kStB);
+        const int pixel = __float_as_int(B.x);
+        const bool first = __float_as_int(A.w) == P.cam.max_depth;
         int pid = -1;
         float t = INF;
-        float3 n = f3(0.0f, 0.0f, 0.0f);
+        Surface sf;
+        sf.n = f3(0.0f, 0.0f, 0.0f), sf.front = false;
         if (h.ref != REF_NONE) {
-          const Surface sf = surface_at(sc, h, o, d, 0.0f);
+          sf = surface_at(sc, h, o, d, 0.0f);
           const uint32_t type = h.ref >> 30, idx = h.ref & 0x3FFFFFFFu;
           if (type == REF_BOX) {  // the reference quad behind this face of the box (scene_build.hpp, box_meta)
             const int4 meta = sc.box_meta[idx >> 3];
@@ -269,11 +277,37 @@ __global__ void __launch_bounds__(kRenderThreads, 1) render_kernel(const __grid_
           } else {
             pid = type == REF_SPHERE ? sc.xspheres[idx].pid : (type == REF_QUAD ? sc.xquads[idx].pid : -2 - int(idx));
           }
-          t = sf.t, n = sf.n;
+          t = sf.t;
         }
-        P.aov_id[pixel] = pid, P.aov_t[pixel] = t;
-        P.aov_n[3 * pixel] = n.x, P.aov_n[3 * pixel + 1] = n.y, P.aov_n[3 * pixel + 2] = n.z;
         alive = false;
+        if (first) {
+          P.aov_id[pixel] = pid, P.aov_t[pixel] = t;
+          P.aov_n[3 * pixel] = sf.n.x, P.aov_n[3 * pixel + 1] = sf.n.y, P.aov_n[3 * pixel + 2] = sf.n.z;
+          if (P.aov_b) {
+            float* r = P.aov_b + kAovBounce * pixel;
+            bool cont = false;
+            float3 d_out = f3(0.0f, 0.0f, 0.0f);
+            if (h.ref != REF_NONE) {  // the shade of rt_render's first segment (below), sample 0
+              const uint4 rnd = rng_block(PathKey{P.key, uint32_t(pixel), uint32_t(__float_as_int(B.y) - 1)}, 1u, 0u);
+              float3 emit, atten;
+              cont = scatter_ray<false>(sc, sf, d, rnd, emit, atten, d_out, nullptr);
+            }
+            for (int k = 0; k < kAovBounce; k++) r[k] = 0.0f;
+            r[10] = __int_as_float(RT_NO_BOUNCE);
+            if (cont) {
+              o = sf.p;
+              d = d_out;
+              r[0] = o.x, r[1] = o.y, r[2] = o.z, r[3] = d.x, r[4] = d.y, r[5] = d.z;
+              const uint32_t skip = (h.ref >> 30) == REF_MEDIUM ? REF_NONE : h.ref;
+              sts_f4(st_a, make_float4(A.x, A.y, A.z, __int_as_float(__float_as_int(A.w) - 1)));
+              asm volatile("st.shared.u32 [%0], %1;" ::"r"(st_a + kStB + 12u), "r"(skip) : "memory");
+              alive = true;
+            }
+          }
+        } else {
+          float* r = P.aov_b + kAovBounce * pixel;
+          r[6] = sf.n.x, r[7] = sf.n.y, r[8] = sf.n.z, r[9] = t, r[10] = __int_as_float(pid), r[11] = sf.front ? 1.0f : 0.0f;
+        }
       }
       continue;
     }
@@ -374,6 +408,7 @@ struct TraceParams {
   const double* origin;
   const double* direction;
   const double* time;
+  const uint32_t* skip;  // fp32 mode: the device ref each ray starts on (rt_trace_rays_from), NULL = none
   double tmin, tmax;
   int flags;
   unsigned long long seed;
@@ -488,7 +523,7 @@ __global__ void __launch_bounds__(256) trace_kernel(const __grid_constant__ Trac
     PathKey key{make_uint2((unsigned)P.seed, (unsigned)(P.seed >> 32)), (uint32_t)i, 0u};
     bool media = sc.n_media && !(P.flags & RT_TRACE_SKIP_MEDIA);
     float tmaxf = P.tmax < 3e38 ? float(P.tmax) : __int_as_float(0x7f800000);
-    Hit h = closest_hit<false>(sc, ns, o, d, float(tm), float(P.tmin), tmaxf, REF_NONE, media, key, 1u, nullptr);
+    Hit h = closest_hit<false>(sc, ns, o, d, float(tm), float(P.tmin), tmaxf, P.skip ? P.skip[i] : REF_NONE, media, key, 1u, nullptr);
     if (h.ref != REF_NONE) {
       Surface sf = surface_at(sc, h, o, d, float(tm));
       uint32_t type = h.ref >> 30, idx = h.ref & 0x3FFFFFFFu;
@@ -592,10 +627,11 @@ struct rt_ctx {
   // created: rt_render itself never looks at the environment, its behaviour is a function of its arguments and the context.
   //   RT_B200_KERNEL=mega|stream|refill  default render kernel        RT_B200_NO_STAGING=1   BVH top levels only in shared memory
   //   RT_B200_CHUNK_MAX=n                samples per work item <= n   RT_B200_MAX_CHUNKS=n   launches of <= n sample chunks (test hook)
+  //   RT_B200_NO_SMEM_STACK=1            megakernel traversal stacks in local memory (test hook: every plan under one scene)
   struct Knobs {
     int kernel = 0;
     int chunk_max = 0, max_chunks = 0;
-    bool no_staging = false;
+    bool no_staging = false, no_smem_stack = false;
   } knobs;
   cudaStream_t stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -721,13 +757,13 @@ struct Scratch {
   }
 };
 
-int run_trace(rt_ctx* ctx, long long n, const double* d_origin, const double* d_dir, const double* d_time, double tmin, double tmax, int flags,
-              int32_t* prim_id, double* t, double* normal, uint8_t* front_face, Scratch& sx) {
+int run_trace(rt_ctx* ctx, long long n, const double* d_origin, const double* d_dir, const double* d_time, const uint32_t* d_skip, double tmin, double tmax,
+              int flags, int32_t* prim_id, double* t, double* normal, uint8_t* front_face, Scratch& sx) {
   TraceParams P;
   std::memset(&P, 0, sizeof P);
   P.sc = ctx->sc;
   P.n = n;
-  P.origin = d_origin, P.direction = d_dir, P.time = d_time;
+  P.origin = d_origin, P.direction = d_dir, P.time = d_time, P.skip = d_skip;
   P.tmin = tmin, P.tmax = tmax, P.flags = flags, P.seed = 0;
   P.prim_id = prim_id ? sx.alloc<int>(size_t(n)) : nullptr;
   P.t = t ? sx.alloc<double>(size_t(n)) : nullptr;
@@ -747,6 +783,50 @@ int run_trace(rt_ctx* ctx, long long n, const double* d_origin, const double* d_
   if (t) RT_CUDA(ctx, cudaMemcpy(t, P.t, size_t(n) * 8, cudaMemcpyDeviceToHost));
   if (normal) RT_CUDA(ctx, cudaMemcpy(normal, P.normal, size_t(n) * 24, cudaMemcpyDeviceToHost));
   if (front_face) RT_CUDA(ctx, cudaMemcpy(front_face, P.front, size_t(n), cudaMemcpyDeviceToHost));
+  return RT_OK;
+}
+
+// Reference primitive id -> the device ref a ray that starts on it carries into the traversal (the `skip` rt_render sets
+// after a scatter): a sphere or quad of the BVH is its own ref; a quad of a box() list is that box with the face bits
+// (box_meta's face -> quad nibbles, inverted).  Only primitives the BVH references have one; an id that names two
+// different device primitives (a hittable reached twice through the graph) cannot be resolved.  Both are refused.
+int start_refs(rt_ctx* ctx, long long n, const int32_t* start_prim, std::vector<uint32_t>& out) {
+  const HostScene& h = ctx->host;
+  std::vector<uint32_t> ref_of;  // indexed by reference primitive id
+  auto add = [&](int pid, uint32_t ref) {
+    if (pid < 0) return true;
+    if (size_t(pid) >= ref_of.size()) ref_of.resize(size_t(pid) + 1, REF_NONE);
+    if (ref_of[size_t(pid)] != REF_NONE && ref_of[size_t(pid)] != ref) return false;
+    ref_of[size_t(pid)] = ref;
+    return true;
+  };
+  for (uint32_t ref : h.leaf_refs) {
+    if (ref == REF_NONE) continue;
+    const uint32_t type = ref >> 30, idx = ref & 0x3FFFFFFFu;
+    bool ok = true;
+    if (type == REF_SPHERE) {
+      ok = add(h.xspheres[idx].pid, ref);
+    } else if (type == REF_QUAD) {
+      ok = add(h.xquads[idx].pid, ref);
+    } else if (type == REF_BOX) {
+      const uint32_t b = idx >> 3;
+      const int4 meta = h.box_meta[b];
+      for (uint32_t f = 0; f < 6 && ok; f++)
+        ok = add(h.xquads[size_t(meta.y) + ((uint32_t(meta.z) >> (4u * f)) & 7u)].pid, make_ref(REF_BOX, (b << 3) | f));
+    }
+    if (!ok) return fail(ctx, RT_ERR_INVALID, "start_prim: a primitive id names more than one device primitive");
+  }
+  out.resize(size_t(n));
+  for (long long i = 0; i < n; i++) {
+    const int32_t pid = start_prim[i];
+    if (pid == -1) {
+      out[size_t(i)] = REF_NONE;
+    } else if (pid < 0 || size_t(pid) >= ref_of.size() || ref_of[size_t(pid)] == REF_NONE) {
+      return fail(ctx, RT_ERR_INVALID, "start_prim[" + std::to_string(i) + "] = " + std::to_string(pid) + " is not a primitive of the traversal");
+    } else {
+      out[size_t(i)] = ref_of[size_t(pid)];
+    }
+  }
   return RT_OK;
 }
 }  // namespace
@@ -844,6 +924,7 @@ int rt_init(int device, rt_ctx** out) {
   if (const char* k = std::getenv("RT_B200_CHUNK_MAX")) ctx->knobs.chunk_max = std::max(1, std::atoi(k));
   if (const char* k = std::getenv("RT_B200_MAX_CHUNKS")) ctx->knobs.max_chunks = std::max(1, std::atoi(k));
   ctx->knobs.no_staging = std::getenv("RT_B200_NO_STAGING") != nullptr;
+  ctx->knobs.no_smem_stack = std::getenv("RT_B200_NO_SMEM_STACK") != nullptr;
   if ((e = cudaSetDevice(device)) != cudaSuccess) return bail("cudaSetDevice", e);
   lap("cudaSetDevice");
   // two attributes, not cudaGetDeviceProperties: the full property query costs tens of milliseconds (it reads clocks
@@ -1024,7 +1105,7 @@ static MegaPlan plan_megakernel(const rt_ctx* ctx, RenderParams& P) {
   // data: +2..3 % on bouncing_spheres / book1_final (40 KB staged), but -1.4..-7 % on book2_final, whose 127 KB staged
   // BVH + 50 KB of stacks would leave L1 23 KB (gpurun_out/ab_ss1.log).
   const size_t stack_bytes = size_t(std::max(1, ctx->host.bvh_depth)) * 4 * kRenderThreads;
-  mp.sstack = mp.all_smem && RT_SMEM_STACK && ctx->sc.n_nodes <= kSmemStackMaxCode && ((ctx->sc.n_leaf_refs << 3) | 7) <= kSmemStackMaxCode &&
+  mp.sstack = mp.all_smem && RT_SMEM_STACK && !ctx->knobs.no_smem_stack && ctx->sc.n_nodes <= kSmemStackMaxCode && ((ctx->sc.n_leaf_refs << 3) | 7) <= kSmemStackMaxCode &&
               smem + stack_bytes <= kSmemStackBudget && smem + stack_bytes + 4096 <= ctx->smem_optin;
   if (mp.sstack) P.stack_off = unsigned(smem), P.stack_levels = unsigned(std::max(1, ctx->host.bvh_depth)), smem += stack_bytes;
   mp.smem = smem;
@@ -1472,17 +1553,96 @@ int rt_get_stats(rt_ctx* ctx, rt_stats* out) {
 
 int rt_trace_rays(rt_ctx* ctx, int64_t n, const double* origin, const double* direction, const double* time, double tmin, double tmax, int32_t flags,
                   int32_t* prim_id, double* t, double* normal, uint8_t* front_face) {
+  return rt_trace_rays_from(ctx, n, origin, direction, time, nullptr, tmin, tmax, flags, prim_id, t, normal, front_face);
+}
+
+int rt_trace_rays_from(rt_ctx* ctx, int64_t n, const double* origin, const double* direction, const double* time, const int32_t* start_prim, double tmin,
+                       double tmax, int32_t flags, int32_t* prim_id, double* t, double* normal, uint8_t* front_face) {
   if (!ctx) return RT_ERR_INVALID;
   DebugScope dbg("rt_trace_rays");
   if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_trace_rays before rt_upload_scene");
   if (n < 0 || (n > 0 && (!origin || !direction))) return fail(ctx, RT_ERR_INVALID, "bad ray arrays");
+  if (start_prim && (flags & RT_TRACE_EXACT))
+    return fail(ctx, RT_ERR_INVALID, "RT_TRACE_EXACT follows the reference, which has no start primitive: start_prim is for the fp32 traversal");
+  std::vector<uint32_t> skip;
+  if (start_prim) {
+    int rc = start_refs(ctx, n, start_prim, skip);
+    if (rc != RT_OK) return rc;
+  }
   RT_CUDA(ctx, cudaSetDevice(ctx->device));
   Scratch sx;
   const double* d_o = sx.to_device(origin, size_t(3 * n));
   const double* d_d = sx.to_device(direction, size_t(3 * n));
   const double* d_t = sx.to_device(time, size_t(n));
-  if (n > 0 && (!d_o || !d_d || (time && !d_t))) return fail(ctx, RT_ERR_CUDA, "cudaMalloc / copy of the rays failed");
-  return run_trace(ctx, n, d_o, d_d, d_t, tmin, tmax, flags, prim_id, t, normal, front_face, sx);
+  const uint32_t* d_s = start_prim ? sx.to_device(skip.data(), size_t(n)) : nullptr;
+  if (n > 0 && (!d_o || !d_d || (time && !d_t) || (start_prim && !d_s))) return fail(ctx, RT_ERR_CUDA, "cudaMalloc / copy of the rays failed");
+  return run_trace(ctx, n, d_o, d_d, d_t, d_s, tmin, tmax, flags, prim_id, t, normal, front_face, sx);
+}
+
+// The pixel-centre rays through render_kernel itself (its AOV instantiation), planned exactly as rt_render plans it for
+// this scene: same staging, same node form, same stack.  `bounce`: also the second segment (P.aov_b).  Host outputs:
+// prim_id, t (n), normal (3n), rec (kAovBounce n); prim_id and rec may be NULL.
+static int render_aov(rt_ctx* ctx, const rt_camera_desc* cam, const rt_camera_frame& f, uint64_t seed, bool bounce, int32_t* prim_id, float* t, float* normal,
+                      float* rec) {
+  const long long n = (long long)f.image_width * f.image_height;
+  Scratch sx;
+  RenderParams P;
+  std::memset(&P, 0, sizeof P);
+  P.sc = ctx->sc;
+  fill_camera(cam, f, P.cam);
+  P.cam.max_depth = bounce ? 2 : 1;
+  P.key = make_uint2((unsigned)seed, (unsigned)(seed >> 32));
+  P.sample_begin = 0, P.sample_count = 1, P.chunk = 1, P.n_chunks = 1;
+  P.tiles_x = (f.image_width + 7) / 8, P.tiles_y = (f.image_height + 3) / 4;
+  const unsigned long long n_items = (unsigned long long)P.tiles_x * P.tiles_y * 32ull;
+  if (n_items >= 0xFFFFFFFFull - (unsigned long long)ctx->sm_count * kRenderThreads) return fail(ctx, RT_ERR_INVALID, "image too large");
+  P.per_chunk = unsigned(n_items), P.n_items = unsigned(n_items);
+  P.counters = sx.alloc<unsigned long long>(32);
+  P.aov_id = sx.alloc<int>(size_t(n));
+  P.aov_t = sx.alloc<float>(size_t(n));
+  P.aov_n = sx.alloc<float>(size_t(3 * n));
+  P.aov_b = bounce ? sx.alloc<float>(size_t(kAovBounce * n)) : nullptr;
+  if (!P.counters || !P.aov_id || !P.aov_t || !P.aov_n || (bounce && !P.aov_b)) return fail(ctx, RT_ERR_CUDA, "cudaMalloc failed");
+  RT_CUDA(ctx, cudaMemsetAsync(P.counters, 0, 32 * sizeof(unsigned long long), ctx->stream));
+  const MegaPlan mp = plan_megakernel(ctx, P);
+  void (*kern)(RenderParams) = mp.sstack ? render_kernel<false, true, true, true> : (mp.all_smem ? render_kernel<false, true, false, true> : render_kernel<false, false, false, true>);
+  RT_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(mp.smem)));
+  RT_CUDA(ctx, launch_render(kern, ctx->sm_count, mp.smem, ctx->stream, P));
+  ctx->launches++;
+  RT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if (prim_id) RT_CUDA(ctx, cudaMemcpy(prim_id, P.aov_id, size_t(n) * 4, cudaMemcpyDeviceToHost));
+  RT_CUDA(ctx, cudaMemcpy(t, P.aov_t, size_t(n) * 4, cudaMemcpyDeviceToHost));
+  RT_CUDA(ctx, cudaMemcpy(normal, P.aov_n, size_t(3 * n) * 4, cudaMemcpyDeviceToHost));
+  if (rec) RT_CUDA(ctx, cudaMemcpy(rec, P.aov_b, size_t(kAovBounce * n) * 4, cudaMemcpyDeviceToHost));
+  return RT_OK;
+}
+
+int rt_bounce_visibility(rt_ctx* ctx, const rt_camera_desc* cam, uint64_t seed, int32_t* prim_id, double* t, float* origin1, float* dir1, int32_t* bounce_id,
+                         double* bounce_t, double* bounce_normal, uint8_t* bounce_front) {
+  if (!ctx) return RT_ERR_INVALID;
+  DebugScope dbg("rt_bounce_visibility");
+  if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_bounce_visibility before rt_upload_scene");
+  if (!cam || cam->image_width <= 0 || !(cam->aspect_ratio > 0)) return fail(ctx, RT_ERR_INVALID, "bad camera");
+  RT_CUDA(ctx, cudaSetDevice(ctx->device));
+  rt_camera_frame f;
+  rt_camera_initialize(cam, &f);
+  const size_t n = size_t(f.image_width) * size_t(f.image_height);
+  std::vector<float> ht(n), hn(3 * n), rec(kAovBounce * n);
+  int rc = render_aov(ctx, cam, f, seed, true, prim_id, ht.data(), hn.data(), rec.data());
+  if (rc != RT_OK) return rc;
+  for (size_t i = 0; i < n; i++) {
+    const float* r = rec.data() + kAovBounce * i;
+    if (t) t[i] = double(ht[i]);
+    for (int k = 0; k < 3; k++) {
+      if (origin1) origin1[3 * i + k] = r[k];
+      if (dir1) dir1[3 * i + k] = r[3 + k];
+      if (bounce_normal) bounce_normal[3 * i + k] = double(r[6 + k]);
+    }
+    if (bounce_t) bounce_t[i] = double(r[9]);
+    if (bounce_id) bounce_id[i] = __builtin_bit_cast(int32_t, r[10]);
+    if (bounce_front) bounce_front[i] = r[11] != 0.0f;
+  }
+  return RT_OK;
 }
 
 int rt_primary_visibility(rt_ctx* ctx, const rt_camera_desc* cam, int32_t flags, int32_t* prim_id, double* t, double* normal) {
@@ -1496,35 +1656,10 @@ int rt_primary_visibility(rt_ctx* ctx, const rt_camera_desc* cam, int32_t flags,
   const long long n = (long long)f.image_width * f.image_height;
   Scratch sx;
   if (flags & RT_TRACE_RENDER_KERNEL) {
-    // the pixel-centre rays go through render_kernel itself (its AOV instantiation), planned exactly as rt_render plans
-    // it for this scene: same staging, same node form, same stack
     if (flags & RT_TRACE_EXACT) return fail(ctx, RT_ERR_INVALID, "RT_TRACE_RENDER_KERNEL is the fp32 production traversal: not with RT_TRACE_EXACT");
-    RenderParams P;
-    std::memset(&P, 0, sizeof P);
-    P.sc = ctx->sc;
-    fill_camera(cam, f, P.cam);
-    P.cam.max_depth = 1;
-    P.sample_begin = 0, P.sample_count = 1, P.chunk = 1, P.n_chunks = 1;
-    P.tiles_x = (f.image_width + 7) / 8, P.tiles_y = (f.image_height + 3) / 4;
-    const unsigned long long n_items = (unsigned long long)P.tiles_x * P.tiles_y * 32ull;
-    if (n_items >= 0xFFFFFFFFull - (unsigned long long)ctx->sm_count * kRenderThreads) return fail(ctx, RT_ERR_INVALID, "image too large");
-    P.per_chunk = unsigned(n_items), P.n_items = unsigned(n_items);
-    P.counters = sx.alloc<unsigned long long>(32);
-    P.aov_id = sx.alloc<int>(size_t(n));
-    P.aov_t = sx.alloc<float>(size_t(n));
-    P.aov_n = sx.alloc<float>(size_t(3 * n));
-    if (!P.counters || !P.aov_id || !P.aov_t || !P.aov_n) return fail(ctx, RT_ERR_CUDA, "cudaMalloc failed");
-    RT_CUDA(ctx, cudaMemsetAsync(P.counters, 0, 32 * sizeof(unsigned long long), ctx->stream));
-    const MegaPlan mp = plan_megakernel(ctx, P);
-    void (*kern)(RenderParams) = mp.sstack ? render_kernel<false, true, true, true> : (mp.all_smem ? render_kernel<false, true, false, true> : render_kernel<false, false, false, true>);
-    RT_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(mp.smem)));
-    RT_CUDA(ctx, launch_render(kern, ctx->sm_count, mp.smem, ctx->stream, P));
-    ctx->launches++;
-    RT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     std::vector<float> ht(static_cast<size_t>(n)), hn(static_cast<size_t>(3 * n));
-    if (prim_id) RT_CUDA(ctx, cudaMemcpy(prim_id, P.aov_id, size_t(n) * 4, cudaMemcpyDeviceToHost));
-    RT_CUDA(ctx, cudaMemcpy(ht.data(), P.aov_t, size_t(n) * 4, cudaMemcpyDeviceToHost));
-    RT_CUDA(ctx, cudaMemcpy(hn.data(), P.aov_n, size_t(3 * n) * 4, cudaMemcpyDeviceToHost));
+    int rc = render_aov(ctx, cam, f, 0, false, prim_id, ht.data(), hn.data(), nullptr);
+    if (rc != RT_OK) return rc;
     if (t)
       for (long long i = 0; i < n; i++) t[i] = double(ht[size_t(i)]);
     if (normal)
@@ -1538,7 +1673,7 @@ int rt_primary_visibility(rt_ctx* ctx, const rt_camera_desc* cam, int32_t flags,
   center_rays_kernel<<<grid, 128, 0, ctx->stream>>>(f, d_o, d_d);
   ctx->launches++;
   RT_CUDA(ctx, cudaGetLastError());
-  return run_trace(ctx, n, d_o, d_d, nullptr, 0.001, INFINITY, flags, prim_id, t, normal, nullptr, sx);
+  return run_trace(ctx, n, d_o, d_d, nullptr, nullptr, 0.001, INFINITY, flags, prim_id, t, normal, nullptr, sx);
 }
 
 int rt_medium_spans(rt_ctx* ctx, int32_t medium_index, int64_t n, const double* origin, const double* direction, const double* time, double* t1,

@@ -8,34 +8,7 @@ import scene_util as su
 pytestmark = pytest.mark.gpu
 
 
-def random_scene(rng, n_spheres=40, n_quads=40, n_boxes=6):
-    s = su.SceneDesc()
-    mat = s.lambertian(s.solid(0.5, 0.5, 0.5))
-    kids = []
-    for _ in range(n_spheres):
-        c = rng.uniform(-10, 10, 3)
-        c2 = c + rng.uniform(-1, 1, 3) if rng.random() < 0.4 else None
-        kids.append(s.sphere(tuple(c), float(rng.uniform(0.2, 2.5)), mat, None if c2 is None else tuple(c2)))
-    for _ in range(n_quads):
-        kids.append(s.quad(tuple(rng.uniform(-10, 10, 3)), tuple(rng.uniform(-4, 4, 3)), tuple(rng.uniform(-4, 4, 3)), mat))
-    for _ in range(n_boxes):
-        b = s.box(tuple(rng.uniform(-2, 0, 3)), tuple(rng.uniform(0.5, 3, 3)), mat)
-        b = s.rotate_y(b, float(rng.uniform(-80, 80)))
-        b = s.translate(b, tuple(rng.uniform(-8, 8, 3)))
-        if rng.random() < 0.5:  # nested wrappers
-            b = s.translate(s.rotate_y(b, float(rng.uniform(-30, 30))), tuple(rng.uniform(-2, 2, 3)))
-        kids.append(b)
-    # instanced moving spheres
-    sub = s.list([s.sphere(tuple(rng.uniform(-1, 1, 3)), 0.5, mat, tuple(rng.uniform(-1, 1, 3))) for _ in range(5)])
-    kids.append(s.translate(s.rotate_y(sub, 33.0), (3.0, -2.0, 1.0)))
-    return s, s.finish(s.list(kids))
-
-
-def random_rays(rng, n):
-    o = rng.uniform(-14, 14, (n, 3))
-    target = rng.uniform(-9, 9, (n, 3))
-    d = (target - o) * rng.uniform(0.05, 3.0, (n, 1))  # un-normalised, like the reference's rays
-    return o, d, rng.uniform(0, 1, n)
+random_scene, random_rays = su.random_scene, su.random_rays
 
 
 @pytest.mark.parametrize("seed", [1, 2, 3])

@@ -38,6 +38,12 @@ for name, depth in (("book2_final", 40), ("cornell_smoke", 50), ("bouncing_spher
     d = rng.normal(size=(n, 3))
     ctx.trace_rays(o, d, rng.uniform(0, 1, n), 0.001, np.inf, rtb.RT_TRACE_FP32)
     ctx.trace_rays(o, d, None, 0.001, np.inf, rtb.RT_TRACE_EXACT)
+    # bounce rays: the start-primitive rules of the fp32 traversal, and the render kernel's own second segment
+    ids0 = ctx.primary_visibility(cam, rtb.RT_TRACE_EXACT | rtb.RT_TRACE_SKIP_MEDIA)[0].reshape(-1)
+    starts = rng.choice(np.unique(ids0[ids0 >= 0]), n)
+    ctx.trace_rays(o, d, rng.uniform(0, 1, n), 0.001, np.inf, rtb.RT_TRACE_FP32, start_prim=starts)
+    b = ctx.bounce_visibility(cam, seed=9)
+    assert (b["id"] == ids["render"]).all()
     # every render kernel, same bits
     acc = {}
     for tag, flags in (("mega", rtb.RT_RENDER_MEGAKERNEL), ("stream", rtb.RT_RENDER_STREAM), ("refill", rtb.RT_RENDER_REFILL),
