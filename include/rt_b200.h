@@ -232,9 +232,29 @@ enum {
  * sums per pixel: integer addition is associative, so the image is bit-identical for
  * any sharding of the samples over ranks / GPUs / launches.                            */
 int rt_render(rt_ctx* ctx, const rt_camera_desc* cam, const rt_render_opts* opts);
+
+/* n_views camera views of the uploaded scene in ONE launch: a turntable, the frames of an
+ * animation, a multi-view dataset.  View v of the accumulator gets exactly the bits
+ * rt_render(&cams[v], opts) gives (same Philox stream: the counter is the in-view pixel,
+ * sample and bounce).  The accumulator becomes n_views x H x W x 3 int64, view-major;
+ * rt_download and rt_accum_device_ptr return the whole batch, and rt_stats.n_views says
+ * how many images it holds.  A later rt_render / rt_upload_accum makes it one image again.
+ *   - Every camera has the same image_width, image height (as rt_camera_initialize
+ *     computes it) and samples_per_pixel; every other field (lookfrom / lookat / vup,
+ *     vfov, defocus, max_depth, background) may differ per view.  A view with
+ *     max_depth <= 0 traces nothing, as rt_render; its samples still count in stats.
+ *   - opts: seed, sample_begin / sample_count and clear mean what they mean for rt_render;
+ *     one seed serves all views.  Always the megakernel (RT_B200_KERNEL does not apply).
+ *   - RT_ERR_INVALID: n_views < 1, NULL cams / opts, a camera rt_render refuses, views of
+ *     different sizes or spp, an empty sample range, n_views x W x H > INT32_MAX.
+ *     RT_ERR_UNSUPPORTED: peer_accum, push_accum, RT_RENDER_COUNTERS, RT_RENDER_STREAM,
+ *     RT_RENDER_REFILL (across GPUs, shard a batch by views).  RT_ERR_NO_SCENE.
+ * Asynchronous like rt_render; more than 2^32 work items are split over sample ranges. */
+int rt_render_views(rt_ctx* ctx, int32_t n_views, const rt_camera_desc* cams, const rt_render_opts* opts);
 int rt_synchronize(rt_ctx* ctx);
 
-/* The accumulator (3 x int64 per pixel, row-major from the top-left, interleaved RGB)
+/* The accumulator (3 x int64 per pixel, row-major from the top-left, interleaved RGB;
+ * after rt_render_views, one such image per view, view-major)
  * as a raw device pointer, for the multi-GPU reduce (NCCL ncclInt64 sum, or peer adds). */
 int rt_accum_device_ptr(rt_ctx* ctx, void** dev_ptr, size_t* bytes);
 
@@ -263,7 +283,8 @@ typedef enum rt_buffer_kind {
 } rt_buffer_kind;
 
 /* Synchronises and copies the image to host memory.  samples_per_pixel is the total
- * number of samples accumulated (over all ranks) and only scales F32 / RGB8 output.    */
+ * number of samples accumulated (over all ranks) and only scales F32 / RGB8 output.
+ * After rt_render_views every kind holds the whole batch, view-major (n_views images). */
 int rt_download(rt_ctx* ctx, rt_buffer_kind kind, int32_t samples_per_pixel, void* dst,
                 size_t bytes);
 
@@ -287,7 +308,8 @@ typedef struct rt_stats {
   int32_t bvh_nodes_in_smem;
   int32_t kernel_launches; /* number of kernels this context has launched              */
   int32_t n_boxes;         /* box() lists turned into one slab-test primitive each     */
-  int32_t reserved0;
+  int32_t n_views;         /* images the accumulator holds: 1 after rt_render / rt_upload_accum,
+                              n_views after rt_render_views, 0 before anything was rendered */
   /* RT_RENDER_COUNTERS only, since the last clear — the N_* of the roofline model:
    * [0] BVH node visits (2 box tests each) [1] sphere tests [2] sphere hits [3] quad tests
    * [4] quad tests past the plane/t early-outs [5] medium tests [6..10] scatters by material

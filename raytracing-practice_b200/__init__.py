@@ -51,6 +51,7 @@ def cuda_lib():
         lib.rt_shutdown.restype = None
         lib.rt_upload_scene.argtypes = [C.c_void_p, C.POINTER(_abi.rt_scene_desc)]
         lib.rt_render.argtypes = [C.c_void_p, C.POINTER(_abi.rt_camera_desc), C.POINTER(_abi.rt_render_opts)]
+        lib.rt_render_views.argtypes = [C.c_void_p, C.c_int32, C.POINTER(_abi.rt_camera_desc), C.POINTER(_abi.rt_render_opts)]
         lib.rt_synchronize.argtypes = [C.c_void_p]
         lib.rt_accum_device_ptr.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t)]
         lib.rt_reduce_buffer.argtypes = [C.c_void_p, C.POINTER(_abi.rt_camera_desc), C.POINTER(C.c_void_p), C.POINTER(_abi.rt_ipc_handle)]
@@ -165,6 +166,7 @@ class Context:
         if rc != RT_OK:
             raise RtError(f"rt_init({device}) failed ({rc}): {self._lib.rt_last_error(None).decode()}")
         self.device = device
+        self._views = False  # the accumulator holds a batch of rt_render_views: downloads are (V, H, W, 3)
 
     def _check(self, rc, what):
         if rc != RT_OK:
@@ -175,7 +177,18 @@ class Context:
 
     def render(self, cam, seed=0, sample_begin=0, sample_count=0, clear=True, peer_accum=None, flags=0, push_accum=None):
         o = _abi.rt_render_opts(seed, sample_begin, sample_count, 1 if clear else 0, flags, peer_accum, push_accum)
+        self._views = False
         self._check(self._lib.rt_render(self._h, C.byref(cam), C.byref(o)), "rt_render")
+
+    def render_views(self, cams, seed=0, sample_begin=0, sample_count=0, clear=True, flags=0):
+        """Render several views of the uploaded scene in one launch (rt_render_views).  `cams`: a sequence of
+        rt_camera_desc of one image size and spp.  View v gets the bits render(cams[v], seed, ...) gives; the downloads
+        then return (V, H, W, 3)."""
+        cams = list(cams)
+        arr = (_abi.rt_camera_desc * max(len(cams), 1))(*cams)
+        o = _abi.rt_render_opts(seed, sample_begin, sample_count, 1 if clear else 0, flags, None, None)
+        self._check(self._lib.rt_render_views(self._h, len(cams), arr if cams else None, C.byref(o)), "rt_render_views")
+        self._views = True
 
     def reduce_buffer(self, cam):
         """Allocate / zero this context's reduce buffer for `cam`; returns (device pointer, 64-byte IPC handle)."""
@@ -224,22 +237,26 @@ class Context:
         self._check(self._lib.rt_download(self._h, kind, spp, arr.ctypes.data_as(C.c_void_p), arr.nbytes), "rt_download")
         return arr
 
-    def download_accum(self):
+    def _image_shape(self):
+        """(H, W, 3) after render / upload_accum; (V, H, W, 3) after render_views, also for V = 1."""
         s = self.stats()
-        return self._download(RT_BUF_ACCUM_I64, 1, np.empty((s.image_height, s.image_width, 3), np.int64))
+        shape = (s.image_height, s.image_width, 3)
+        return (s.n_views,) + shape if self._views or s.n_views > 1 else shape
+
+    def download_accum(self):
+        return self._download(RT_BUF_ACCUM_I64, 1, np.empty(self._image_shape(), np.int64))
 
     def upload_accum(self, cam, sums):
         """Replace the accumulator with saved int64 sums (H x W x 3): the inverse of download_accum."""
         a = np.ascontiguousarray(sums, dtype=np.int64)
+        self._views = False
         self._check(self._lib.rt_upload_accum(self._h, C.byref(cam), a.ctypes.data_as(C.c_void_p), a.nbytes), "rt_upload_accum")
 
     def download_radiance(self, spp):
-        s = self.stats()
-        return self._download(RT_BUF_RADIANCE_F32, spp, np.empty((s.image_height, s.image_width, 3), np.float32))
+        return self._download(RT_BUF_RADIANCE_F32, spp, np.empty(self._image_shape(), np.float32))
 
     def download_rgb8(self, spp):
-        s = self.stats()
-        return self._download(RT_BUF_RGB8, spp, np.empty((s.image_height, s.image_width, 3), np.uint8))
+        return self._download(RT_BUF_RGB8, spp, np.empty(self._image_shape(), np.uint8))
 
     def trace_rays(self, origin, direction, time=None, tmin=0.001, tmax=float("inf"), flags=RT_TRACE_FP32, start_prim=None):
         """start_prim: per ray the primitive id it starts on (-1: none), for rays that leave a surface as rt_render's

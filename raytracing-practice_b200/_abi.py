@@ -155,7 +155,7 @@ class rt_stats(C.Structure):
         ("bvh_nodes_in_smem", C.c_int32),
         ("kernel_launches", C.c_int32),
         ("n_boxes", C.c_int32),
-        ("reserved0", C.c_int32),
+        ("n_views", C.c_int32),
         ("census", C.c_uint64 * 16),
     ]
 
@@ -168,6 +168,7 @@ C_ABI_SYMBOLS = [
     "rt_last_error",
     "rt_upload_scene",
     "rt_render",
+    "rt_render_views",
     "rt_synchronize",
     "rt_accum_device_ptr",
     "rt_reduce_buffer",

@@ -68,6 +68,12 @@ struct RenderParams {
   float* aov_n;
   float* aov_b;            // render_kernel<.., AOV> with max_depth 2: the bounce segment, kAovBounce floats per pixel
   StreamLayout sl;   // streaming kernel only
+  // render_kernel<.., VIEWS> (rt_render_views): one camera per view; `cam` above carries the size all views share.
+  // A work item's global pixel is view * view_pixels + in-view pixel, and per_chunk covers all views.
+  const CameraDev* cams;
+  int n_views;
+  unsigned int view_items;   // work items per view and sample chunk = tiles_x * tiles_y * 32
+  unsigned int view_pixels;  // W * H
 };
 
 #ifndef RT_THREADS
@@ -127,7 +133,12 @@ __global__ void push_kernel(const unsigned long long* __restrict__ accum, unsign
 // is written as the record {origin1.xyz, dir1.xyz, normal.xyz, t, id bits, front}.
 // COOP = true evaluates Perlin turbulence warp-cooperatively (below); chosen per scene by the launch plan — only where a
 // good share of the primitives carries a noise texture: the hoisted hit record it needs costs the other scenes 3 %.
-template <bool COUNT, bool ALL_SMEM, bool SSTACK = false, bool AOV = false, bool COOP = false>
+// VIEWS = true renders a batch of views of one scene (rt_render_views): the work items of a sample chunk run over
+// (view, tile, lane), and a path's global pixel — the one its state record holds — is view * W * H + its in-view pixel.
+// Its camera, its Philox pixel (the in-view one) and its bounce numbering are derived from that index where they are
+// needed, so nothing more is live across the traversal; the sums go to view-major images.  Every path is the path
+// rt_render(cams[view]) traces, so view v has the bits of that render.
+template <bool COUNT, bool ALL_SMEM, bool SSTACK = false, bool AOV = false, bool COOP = false, bool VIEWS = false>
 __global__ void __launch_bounds__(kRenderThreads, 1) render_kernel(const __grid_constant__ RenderParams P) {
   extern __shared__ float4 s_nodes[];
   stage_nodes<ALL_SMEM>(s_nodes, P.sc.nodes, P.smem_nodes);
@@ -147,6 +158,19 @@ __global__ void __launch_bounds__(kRenderThreads, 1) render_kernel(const __grid_
   const NodeSource ns = node_source(s_nodes, P.sc.nodes, P.smem_nodes, P.sc.n_nodes);
   const DeviceScene& sc = P.sc;
   const float INF = __int_as_float(0x7f800000);
+  // the camera of a global pixel index, and its in-view pixel (the pixel of its Philox counter); one camera without VIEWS
+  auto cam_of = [&](int pixel) -> const CameraDev& {
+    if constexpr (VIEWS) {
+      RT_CHECK(unsigned(pixel) / P.view_pixels < unsigned(P.n_views), CHK_VIEW);
+      return P.cams[unsigned(pixel) / P.view_pixels];
+    } else {
+      return P.cam;
+    }
+  };
+  auto view_pixel = [&](int pixel) -> int {
+    if constexpr (VIEWS) return int(unsigned(pixel) % P.view_pixels);
+    else return pixel;
+  };
 
   // Per-lane path state, kept small on purpose: the kernel runs 896 threads per SM (72 registers; 1024 x 64 and 768 x 80
   // are slower, gpurun_out/ab_lean2.log) and it is very sensitive to what is live across the traversal — two more
@@ -202,13 +226,17 @@ __global__ void __launch_bounds__(kRenderThreads, 1) render_kernel(const __grid_
           if (it >= (unsigned long long)P.n_items) break;
           const unsigned int item = (unsigned int)it;
           const unsigned int chunk = item / P.per_chunk, q = item - chunk * P.per_chunk;
-          const unsigned int tile = q >> 5, lane = q & 31u;
+          unsigned int view = 0u, vq = q;  // VIEWS: (view, tile, lane) within the chunk, a warp's 32 items = one tile of one view
+          if constexpr (VIEWS) view = q / P.view_items, vq = q - view * P.view_items;
+          const unsigned int tile = vq >> 5, lane = vq & 31u;
           const int px = int(tile % (unsigned)P.tiles_x) * 8 + int(lane & 7u);
           const int py = int(tile / (unsigned)P.tiles_x) * 4 + int(lane >> 3);
-          if (px < P.cam.W && py < P.cam.H) {
+          // (a view with max_depth <= 0 traces nothing, as rt_render launches nothing for it: its items are skipped)
+          if (px < P.cam.W && py < P.cam.H && (!VIEWS || cam_of(int(view * P.view_pixels)).max_depth > 0)) {
             s = P.sample_begin + int(chunk) * P.chunk;
             if (s < s_last) {
               pixel = py * P.cam.W + px;
+              if constexpr (VIEWS) pixel += int(view * P.view_pixels);
               key.pixel = uint32_t(pixel);
               done = false;
               break;
@@ -219,25 +247,28 @@ __global__ void __launch_bounds__(kRenderThreads, 1) render_kernel(const __grid_
       if (!done) {
         // ---- camera::get_ray (camera.hpp:139-162): jitter, defocus disk, shutter time ----
         key.sample = uint32_t(s++);
-        const int py = pixel / P.cam.W, px = pixel - py * P.cam.W;
+        const CameraDev& cam = cam_of(pixel);
+        const int vpixel = view_pixel(pixel);
+        if constexpr (VIEWS) key.pixel = uint32_t(vpixel);
+        const int py = vpixel / P.cam.W, px = vpixel - py * P.cam.W;
         uint4 r0 = rng_block(key, 0u, 0u);
         float ox = u01(r0.x) - 0.5f, oy = u01(r0.y) - 0.5f;
         float time = u01(r0.z);
         if (AOV) ox = oy = time = 0.0f;
-        float3 dir = fma3(float(px) + ox, P.cam.du, fma3(float(py) + oy, P.cam.dv, P.cam.p00c));
-        o = P.cam.center;
-        if (!AOV && P.cam.defocus) {  // uniform disk: r = sqrt(u), phi = 2 pi v (== rejection sampling in law)
+        float3 dir = fma3(float(px) + ox, cam.du, fma3(float(py) + oy, cam.dv, cam.p00c));
+        o = cam.center;
+        if (!AOV && cam.defocus) {  // uniform disk: r = sqrt(u), phi = 2 pi v (== rejection sampling in law)
           uint4 r1 = rng_block(key, 0u, 1u);
           float rr = sqrtf(u01(r1.x)), sn, cs;
           sincos_2pi(u01(r1.y), sn, cs);
-          float3 off = fma3(rr * cs, P.cam.ddu, (rr * sn) * P.cam.ddv);
+          float3 off = fma3(rr * cs, cam.ddu, (rr * sn) * cam.ddv);
           o = o + off;
           dir = dir - off;
         }
         d = dir;
-        sts_f4(st_a, make_float4(1.0f, 1.0f, 1.0f, __int_as_float(P.cam.max_depth)));
+        sts_f4(st_a, make_float4(1.0f, 1.0f, 1.0f, __int_as_float(cam.max_depth)));
         sts_f4(st_a + kStB, make_float4(__int_as_float(pixel), __int_as_float(s), time, __uint_as_float(REF_NONE)));
-        alive = P.cam.max_depth > 0;
+        alive = cam.max_depth > 0;
       }
     }
     const unsigned live = __ballot_sync(FULL, alive);
@@ -250,8 +281,13 @@ __global__ void __launch_bounds__(kRenderThreads, 1) render_kernel(const __grid_
     // the ray's Philox counter, read back for the scene-enclosing media (every ray) and — lazily — for a medium leaf
     auto key_of = [&](PathKey& k, uint32_t& b) {
       const float4 A = lds_f4(st_a), B = lds_f4(st_a + kStB);
-      k = PathKey{P.key, uint32_t(__float_as_int(B.x)), uint32_t(__float_as_int(B.y) - 1)};
-      b = uint32_t(P.cam.max_depth - __float_as_int(A.w)) + 1u;
+      if constexpr (VIEWS) {
+        k = PathKey{P.key, uint32_t(view_pixel(__float_as_int(B.x))), uint32_t(__float_as_int(B.y) - 1)};
+        b = uint32_t(cam_of(__float_as_int(B.x)).max_depth - __float_as_int(A.w)) + 1u;
+      } else {
+        k = PathKey{P.key, uint32_t(__float_as_int(B.x)), uint32_t(__float_as_int(B.y) - 1)};
+        b = uint32_t(P.cam.max_depth - __float_as_int(A.w)) + 1u;
+      }
     };
     auto aux_of = [&](float& t, uint32_t& sk) {
       float tt, ss;
@@ -333,14 +369,15 @@ __global__ void __launch_bounds__(kRenderThreads, 1) render_kernel(const __grid_
       int depth = __float_as_int(A.w);
       const int pixel = __float_as_int(B.x);
       const float time = B.z;
-      const PathKey key{P.key, uint32_t(pixel), uint32_t(__float_as_int(B.y) - 1)};
-      const uint32_t bounce = uint32_t(P.cam.max_depth - depth) + 1u;
+      const CameraDev& cam = cam_of(pixel);
+      const PathKey key{P.key, uint32_t(view_pixel(pixel)), uint32_t(__float_as_int(B.y) - 1)};
+      const uint32_t bounce = uint32_t(cam.max_depth - depth) + 1u;
       // The radiance of a path is beta x (emission | background) at its LAST vertex: no material of the reference both
       // emits and scatters (diffuse_light::scatter is false, material.hpp:36; every other emitted() is black), so no
       // running sum lives across the traversal.
       float3 L = f3(0.0f, 0.0f, 0.0f);
       if (h.ref == REF_NONE) {
-        L = L + beta * P.cam.bg;
+        L = L + beta * cam.bg;
         alive = false;
       } else {
         const uint4 rnd = rng_block(key, bounce, 0u);
@@ -650,6 +687,14 @@ struct rt_ctx {
   unsigned long long* accum = nullptr;
   size_t accum_values = 0;
   int acc_w = 0, acc_h = 0;
+  int acc_views = 0;  // images the accumulator holds: 1 after rt_render / rt_upload_accum, n_views after rt_render_views
+  // rt_render_views' camera table: one CameraDev per view on the device, filled by a stream-ordered copy from a pinned
+  // buffer that outlives it (ev_cams marks when that copy has read it).  Both only grow: with peer access enabled a
+  // cudaMalloc costs tens of milliseconds.
+  CameraDev* cams_dev = nullptr;
+  CameraDev* cams_host = nullptr;
+  int cams_cap = 0;
+  cudaEvent_t ev_cams = nullptr;
   unsigned long long* counters = nullptr;  // 32 x u64: [0] next item, [1] rays, [2] samples, [4..] census
   unsigned long long rays_total = 0, samples_total = 0;
   int smem_nodes = 0;
@@ -903,6 +948,7 @@ int rt_init(int device, rt_ctx** out) {
     if (ctx->counters) cudaFree(ctx->counters);
     if (ctx->ev0) cudaEventDestroy(ctx->ev0);
     if (ctx->ev1) cudaEventDestroy(ctx->ev1);
+    if (ctx->ev_cams) cudaEventDestroy(ctx->ev_cams);
     if (ctx->stream) cudaStreamDestroy(ctx->stream);
     delete ctx;
     return RT_ERR_CUDA;
@@ -939,6 +985,7 @@ int rt_init(int device, rt_ctx** out) {
   lap("cudaStreamCreate (context)");
   if ((e = cudaEventCreate(&ctx->ev0)) != cudaSuccess) return bail("cudaEventCreate", e);
   if ((e = cudaEventCreate(&ctx->ev1)) != cudaSuccess) return bail("cudaEventCreate", e);
+  if ((e = cudaEventCreateWithFlags(&ctx->ev_cams, cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
   if ((e = cudaMalloc(&ctx->counters, 32 * sizeof(unsigned long long))) != cudaSuccess) return bail("cudaMalloc", e);
   if ((e = cudaMemset(ctx->counters, 0, 32 * sizeof(unsigned long long))) != cudaSuccess) return bail("cudaMemset", e);
   lap("events + counters");
@@ -967,8 +1014,11 @@ void rt_shutdown(rt_ctx* ctx) {
   cudaFree(ctx->reduce_buf);
   cudaFree(ctx->scratch);
   cudaFree(ctx->counters);
+  cudaFree(ctx->cams_dev);
+  cudaFreeHost(ctx->cams_host);
   cudaEventDestroy(ctx->ev0);
   cudaEventDestroy(ctx->ev1);
+  cudaEventDestroy(ctx->ev_cams);
   cudaStreamDestroy(ctx->stream);
   delete ctx;
 }
@@ -1166,14 +1216,15 @@ static bool stream_layout(const rt_ctx* ctx, int bvh_depth, StreamLayout& L) {
   return off + sizeof(RenderParams) + 2048 <= ctx->smem_optin;
 }
 
-static int ensure_accum(rt_ctx* ctx, int W, int H, bool clear) {
-  size_t values = size_t(W) * H * 3;
-  if (values != ctx->accum_values || ctx->acc_w != W) {
+// The accumulator for `views` images of W x H (view-major); any change of shape reallocates it and clears it.
+static int ensure_accum(rt_ctx* ctx, int W, int H, bool clear, int views = 1) {
+  size_t values = size_t(W) * H * 3 * size_t(views);
+  if (values != ctx->accum_values || ctx->acc_w != W || ctx->acc_views != views) {
     cudaFree(ctx->accum);
-    ctx->accum = nullptr, ctx->accum_values = 0, ctx->acc_w = ctx->acc_h = 0;  // a failed cudaMalloc below must not leave the old size behind
+    ctx->accum = nullptr, ctx->accum_values = 0, ctx->acc_w = ctx->acc_h = ctx->acc_views = 0;  // a failed cudaMalloc below must not leave the old size behind
     RT_CUDA(ctx, cudaMalloc(&ctx->accum, values * 8));
     ctx->accum_values = values;
-    ctx->acc_w = W, ctx->acc_h = H;
+    ctx->acc_w = W, ctx->acc_h = H, ctx->acc_views = views;
     clear = true;
   }
   if (clear) {
@@ -1351,6 +1402,126 @@ static int render_range(rt_ctx* ctx, const rt_camera_desc* cam, const rt_render_
   if (last_piece) {
     RT_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
     ctx->timed = true;
+  }
+  return RT_OK;
+}
+
+// One launch of render_kernel<.., VIEWS> over the sample range of `opts` for all views; the camera table is filled by the
+// first piece of a request.  The views were checked by rt_render_views: same W x H (f) and spp.
+static int views_range(rt_ctx* ctx, int32_t n_views, const rt_camera_desc* cams, const rt_camera_frame& f, const rt_render_opts* opts, bool first_piece,
+                       bool last_piece) {
+  RT_CUDA(ctx, cudaSetDevice(ctx->device));
+  const int W = f.image_width, H = f.image_height;
+  int rc = ensure_accum(ctx, W, H, opts->clear != 0, n_views);
+  if (rc != RT_OK) return rc;
+  if (first_piece) RT_CUDA(ctx, cudaEventRecord(ctx->ev0, ctx->stream));
+  if (first_piece) {
+    if (n_views > ctx->cams_cap) {
+      RT_CUDA(ctx, cudaStreamSynchronize(ctx->stream));  // a launch in flight may still read the old table
+      cudaFree(ctx->cams_dev);
+      cudaFreeHost(ctx->cams_host);
+      ctx->cams_dev = nullptr, ctx->cams_host = nullptr, ctx->cams_cap = 0;
+      RT_CUDA(ctx, cudaMalloc(&ctx->cams_dev, size_t(n_views) * sizeof(CameraDev)));
+      RT_CUDA(ctx, cudaHostAlloc(&ctx->cams_host, size_t(n_views) * sizeof(CameraDev), cudaHostAllocDefault));
+      ctx->cams_cap = n_views;
+    } else {
+      RT_CUDA(ctx, cudaEventSynchronize(ctx->ev_cams));  // the previous batch's copy has read the pinned buffer
+    }
+    for (int v = 0; v < n_views; v++) {
+      rt_camera_frame fv;
+      rt_camera_initialize(cams + v, &fv);
+      fill_camera(cams + v, fv, ctx->cams_host[v]);
+    }
+    RT_CUDA(ctx, cudaMemcpyAsync(ctx->cams_dev, ctx->cams_host, size_t(n_views) * sizeof(CameraDev), cudaMemcpyHostToDevice, ctx->stream));
+    RT_CUDA(ctx, cudaEventRecord(ctx->ev_cams, ctx->stream));
+  }
+
+  RenderParams P;
+  std::memset(&P, 0, sizeof P);
+  P.sc = ctx->sc;
+  fill_camera(cams, f, P.cam);  // the size every view shares; the kernel reads each view's camera from P.cams
+  P.key = make_uint2((unsigned)opts->seed, (unsigned)(opts->seed >> 32));
+  P.sample_begin = opts->sample_begin;
+  P.sample_count = opts->sample_count;
+  P.tiles_x = (W + 7) / 8;
+  P.tiles_y = (H + 3) / 4;
+  const int grid = ctx->sm_count;
+  const long long threads = (long long)grid * kRenderThreads;
+  // samples per work item as rt_render chooses them, over the whole batch (the sums do not depend on the choice)
+  const long long total = (long long)n_views * W * H * P.sample_count;
+  long long chunk = total / (threads * 8);
+  const long long chunk_max = ctx->knobs.chunk_max > 0 ? ctx->knobs.chunk_max : 32;
+  P.chunk = int(std::max<long long>(1, std::min<long long>({chunk, chunk_max, (long long)P.sample_count})));
+  while (P.chunk & (P.chunk - 1)) P.chunk &= P.chunk - 1;
+  P.n_chunks = (P.sample_count + P.chunk - 1) / P.chunk;
+  P.view_items = unsigned(P.tiles_x) * unsigned(P.tiles_y) * 32u;
+  const unsigned long long per_chunk = (unsigned long long)P.view_items * (unsigned long long)n_views;
+  const unsigned long long n_items = per_chunk * (unsigned long long)P.n_chunks;
+  if (n_items >= 0xFFFFFFFFull - (unsigned long long)threads) return fail(ctx, RT_ERR_INVALID, "views x image x samples too large for one launch: shard the samples");
+  P.per_chunk = unsigned(per_chunk);
+  P.n_items = unsigned(n_items);
+  P.accum = ctx->accum;
+  P.n_values = (unsigned long long)n_views * W * H * 3ull;
+  P.counters = ctx->counters;
+  P.cams = ctx->cams_dev;
+  P.n_views = n_views;
+  P.view_pixels = unsigned(W) * unsigned(H);
+  // the plan rt_render picks for this scene: the views of a batch take the same staging, stack and turbulence form
+  const MegaPlan mp = plan_megakernel(ctx, P);
+  void (*kern)(RenderParams) = mp.coop_noise ? (mp.sstack ? render_kernel<false, true, true, false, true, true>
+                                                          : (mp.all_smem ? render_kernel<false, true, false, false, true, true> : render_kernel<false, false, false, false, true, true>))
+                                             : (mp.sstack ? render_kernel<false, true, true, false, false, true>
+                                                          : (mp.all_smem ? render_kernel<false, true, false, false, false, true> : render_kernel<false, false, false, false, false, true>));
+  RT_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(mp.smem)));
+  RT_CUDA(ctx, cudaMemsetAsync(ctx->counters, 0, sizeof(unsigned long long), ctx->stream));  // counters[0] = next work item
+  RT_CUDA(ctx, launch_render(kern, grid, mp.smem, ctx->stream, P));
+  ctx->launches++;
+  // every view's samples count, also those of a view with max_depth <= 0 (as rt_render counts them)
+  ctx->samples_total += (unsigned long long)n_views * W * H * P.sample_count;
+  if (last_piece) {
+    RT_CUDA(ctx, cudaEventRecord(ctx->ev1, ctx->stream));
+    ctx->timed = true;
+  }
+  return RT_OK;
+}
+
+int rt_render_views(rt_ctx* ctx, int32_t n_views, const rt_camera_desc* cams, const rt_render_opts* opts) {
+  if (!ctx) return RT_ERR_INVALID;
+  DebugScope dbg("rt_render_views");
+  if (n_views < 1 || !cams || !opts) return fail(ctx, RT_ERR_INVALID, "rt_render_views: n_views < 1, or null cameras / options");
+  rt_camera_frame f;
+  for (int32_t v = 0; v < n_views; v++) {
+    const rt_camera_desc* c = cams + v;
+    if (c->image_width <= 0 || c->samples_per_pixel <= 0 || !(c->aspect_ratio > 0)) return fail(ctx, RT_ERR_INVALID, "bad camera (view " + std::to_string(v) + ")");
+    rt_camera_frame fv;
+    rt_camera_initialize(c, &fv);
+    if (v == 0) {
+      f = fv;
+    } else if (fv.image_width != f.image_width || fv.image_height != f.image_height || c->samples_per_pixel != cams[0].samples_per_pixel) {
+      return fail(ctx, RT_ERR_INVALID, "view " + std::to_string(v) + " differs from view 0 in image size or samples_per_pixel: the views of a batch share both");
+    }
+  }
+  if ((long long)n_views * f.image_width * f.image_height > 0x7FFFFFFFll)
+    return fail(ctx, RT_ERR_INVALID, "n_views x image_width x image_height exceeds 2^31 - 1 (the global pixel index is 32-bit)");
+  if (opts->peer_accum || opts->push_accum) return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views has no peer_accum / push_accum: shard a batch by views");
+  if (opts->flags & (RT_RENDER_COUNTERS | RT_RENDER_STREAM | RT_RENDER_REFILL | RT_RENDER_POOL_REMOVED))
+    return fail(ctx, RT_ERR_UNSUPPORTED, "rt_render_views renders with the megakernel only (no RT_RENDER_COUNTERS / STREAM / REFILL)");
+  if (!ctx->has_scene) return fail(ctx, RT_ERR_NO_SCENE, "rt_render_views before rt_upload_scene");
+  const long long count = opts->sample_count > 0 ? opts->sample_count : (long long)cams[0].samples_per_pixel - opts->sample_begin;
+  if (opts->sample_begin < 0 || count <= 0) return fail(ctx, RT_ERR_INVALID, "empty sample range");
+  // more than 2^32 work items: consecutive sample ranges in stream-ordered launches, as rt_render splits
+  const unsigned long long per_chunk = (unsigned long long)n_views * (unsigned long long)((f.image_width + 7) / 8) * (unsigned long long)((f.image_height + 3) / 4) * 32ull;
+  unsigned long long max_chunks = (0xFFFFFFFFull - (unsigned long long)ctx->sm_count * kRenderThreads - 1ull) / per_chunk;
+  if (ctx->knobs.max_chunks > 0) max_chunks = std::min<unsigned long long>(max_chunks, (unsigned long long)ctx->knobs.max_chunks);  // test hook
+  if (max_chunks == 0) return fail(ctx, RT_ERR_INVALID, "batch too large (more than 2^32 work items per sample)");
+  const long long cap = (long long)std::min<unsigned long long>(max_chunks * 32ull, 1ull << 30);
+  rt_render_opts piece = *opts;
+  for (long long done = 0; done < count; done += cap) {
+    piece.sample_begin = int32_t(opts->sample_begin + done);
+    piece.sample_count = int32_t(std::min(cap, count - done));
+    piece.clear = done == 0 ? opts->clear : 0;
+    int rc = views_range(ctx, n_views, cams, f, &piece, done == 0, done + cap >= count);
+    if (rc != RT_OK) return rc;
   }
   return RT_OK;
 }
@@ -1541,6 +1712,7 @@ int rt_get_stats(rt_ctx* ctx, rt_stats* out) {
   }
   out->image_width = ctx->acc_w;
   out->image_height = ctx->acc_h;
+  out->n_views = ctx->acc_views;
   out->n_nodes = ctx->sc.n_nodes;
   out->n_spheres = ctx->sc.n_spheres;
   out->n_quads = ctx->sc.n_quads;

@@ -43,7 +43,7 @@ __device__ unsigned int g_rt_check_count = 0u;  // checks evaluated (a checks bu
 #endif
 // site codes
 enum : int { CHK_NODE = 1, CHK_STACK_LOCAL = 2, CHK_STACK_SMEM = 3, CHK_LEAF_REF = 4, CHK_SPHERE = 5, CHK_QUAD = 6, CHK_BOX = 7, CHK_MEDIUM = 8, CHK_MATERIAL = 9,
-             CHK_TEXTURE = 10, CHK_TEXEL = 11, CHK_PIXEL = 12, CHK_BREF = 13, CHK_STATE = 14 };
+             CHK_TEXTURE = 10, CHK_TEXEL = 11, CHK_PIXEL = 12, CHK_BREF = 13, CHK_STATE = 14, CHK_VIEW = 15 };
 
 // Big, rarely executed helpers are kept OUT of line (RT_OUTLINE): the fully inlined megakernel was
 // 4,096 SASS instructions = 64 KB, and with 32 resident warps at scattered PCs the top stall was

@@ -1100,6 +1100,45 @@ class context_cache {
   std::vector<entry> slots_;
   std::set<std::pair<int, int>> peers_;
 };
+
+// RT_B200_DEVICES as a list of CUDA ordinals (default {0}), at most `limit` of them (and at least one)
+inline std::vector<int> device_list(int limit) {
+  std::vector<int> devices;
+  const char* env = std::getenv("RT_B200_DEVICES");
+  std::string spec = env ? env : "0";
+  for (size_t pos = 0; pos < spec.size();) {
+    size_t comma = spec.find(',', pos);
+    if (comma == std::string::npos) comma = spec.size();
+    if (comma > pos) devices.push_back(std::atoi(spec.substr(pos, comma - pos).c_str()));
+    pos = comma + 1;
+  }
+  if (devices.empty()) devices.push_back(0);
+  if (int(devices.size()) > limit) devices.resize(size_t(std::max(1, limit)));
+  return devices;
+}
+
+// The scene on every context; several are built and uploaded concurrently (rt_upload_scene is synchronous)
+inline void upload_all(const std::vector<rt_ctx*>& ctx, const rt_scene_desc& sd) {
+  const int R = int(ctx.size());
+  if (R == 1) {
+    int rc = rt_upload_scene(ctx[0], &sd);
+    if (rc != RT_OK) die(ctx[0], "rt_upload_scene", rc);
+    return;
+  }
+  std::vector<int> rcs(size_t(R), RT_OK);
+  std::vector<std::thread> workers;
+  for (int r = 0; r < R; r++) {
+    auto job = [&, r] { rcs[size_t(r)] = rt_upload_scene(ctx[size_t(r)], &sd); };
+    try {
+      workers.emplace_back(job);
+    } catch (const std::system_error&) {
+      job();
+    }
+  }
+  for (std::thread& w : workers) w.join();
+  for (int r = 0; r < R; r++)
+    if (rcs[size_t(r)] != RT_OK) die(ctx[size_t(r)], "rt_upload_scene", rcs[size_t(r)]);
+}
 }  // namespace rtb200
 
 // Environment (the reference's camera has no such fields, and the drop-in keeps its class as it is):
@@ -1118,17 +1157,7 @@ inline void camera::render(std::ostream& output_stream, const hittable& world) {
   auto scene = rtb200::flatten_world(world);
   rt_scene_desc sd = scene->desc();
 
-  std::vector<int> devices;
-  const char* env = std::getenv("RT_B200_DEVICES");
-  std::string spec = env ? env : "0";
-  for (size_t pos = 0; pos < spec.size();) {
-    size_t comma = spec.find(',', pos);
-    if (comma == std::string::npos) comma = spec.size();
-    if (comma > pos) devices.push_back(std::atoi(spec.substr(pos, comma - pos).c_str()));
-    pos = comma + 1;
-  }
-  if (devices.empty()) devices.push_back(0);
-  if (int(devices.size()) > samples_per_pixel) devices.resize(size_t(std::max(1, samples_per_pixel)));
+  std::vector<int> devices = rtb200::device_list(samples_per_pixel);
 
   const int R = int(devices.size());
   rtb200::phase_timer timing;
@@ -1139,24 +1168,7 @@ inline void camera::render(std::ostream& output_stream, const hittable& world) {
   // to render).
   std::vector<rt_ctx*> ctx = rtb200::context_cache::get().acquire_all(devices);
   timing.mark("init");
-  if (R == 1) {
-    int rc = rt_upload_scene(ctx[0], &sd);
-    if (rc != RT_OK) rtb200::die(ctx[0], "rt_upload_scene", rc);
-  } else {  // the BVH build + upload of every device's copy, concurrently (rt_upload_scene is synchronous)
-    std::vector<int> rcs(size_t(R), RT_OK);
-    std::vector<std::thread> workers;
-    for (int r = 0; r < R; r++) {
-      auto job = [&, r] { rcs[size_t(r)] = rt_upload_scene(ctx[size_t(r)], &sd); };
-      try {
-        workers.emplace_back(job);
-      } catch (const std::system_error&) {
-        job();
-      }
-    }
-    for (std::thread& w : workers) w.join();
-    for (int r = 0; r < R; r++)
-      if (rcs[size_t(r)] != RT_OK) rtb200::die(ctx[size_t(r)], "rt_upload_scene", rcs[size_t(r)]);
-  }
+  rtb200::upload_all(ctx, sd);
   timing.mark("upload");
   // Several devices: the exchange step (the per-pixel sum of camera.hpp:61) is done on the devices — every context
   // adds its accumulator into the first one's reduce buffer over peer memory (rt_render_opts.push_accum), no host sum.
@@ -1283,6 +1295,58 @@ inline void camera::render(std::ostream& output_stream, const hittable& world) {
   std::printf("\rDone.                       \n");
   std::fflush(stdout);
 }
+
+namespace rtb200 {
+// Several frames of one world — a turntable, an animation's frames: outs[i] receives the P3 text camera::render writes for
+// *cams[i], and stdout the same progress lines, frame after frame, so the program's output is that of a loop of
+// camera::render calls.  The world is flattened and uploaded once per device; every device of RT_B200_DEVICES renders a
+// contiguous range of the frames in one rt_render_views launch (no reduce: each frame is rendered whole on one device).
+// The cameras must share image_width, image height and samples_per_pixel.  RT_B200_CHECKPOINT / RT_B200_P6 do not apply.
+inline void render_views(const hittable& world, const std::vector<const camera*>& cams, const std::vector<std::ostream*>& outs) {
+  if (cams.size() != outs.size()) {
+    std::fprintf(stderr, "rtb200::render_views: %zu cameras but %zu output streams\n", cams.size(), outs.size());
+    std::exit(1);
+  }
+  if (cams.empty()) return;
+  const int V = int(cams.size());
+  std::vector<rt_camera_desc> desc(cams.size());
+  for (int v = 0; v < V; v++) desc[size_t(v)] = cams[size_t(v)]->desc();
+  rt_camera_frame frame;
+  rt_camera_initialize(&desc[0], &frame);
+  const int spp = desc[0].samples_per_pixel;
+
+  auto scene = flatten_world(world);
+  rt_scene_desc sd = scene->desc();
+  std::vector<int> devices = device_list(V);
+  const int R = int(devices.size());
+  std::vector<rt_ctx*> ctx = context_cache::get().acquire_all(devices);
+  upload_all(ctx, sd);
+
+  const size_t image = size_t(frame.image_width) * frame.image_height * 3;
+  std::vector<uint8_t> rgb(image * size_t(V));
+  for (int r = 0; r < R; r++) {  // asynchronous: all devices render concurrently
+    const int begin = int((int64_t(V) * r) / R), end = int((int64_t(V) * (r + 1)) / R);
+    rt_render_opts o;
+    std::memset(&o, 0, sizeof o);
+    o.seed = 0;
+    o.clear = 1;
+    int rc = rt_render_views(ctx[size_t(r)], end - begin, desc.data() + begin, &o);
+    if (rc != RT_OK) die(ctx[size_t(r)], "rt_render_views", rc);
+  }
+  for (int r = 0; r < R; r++) {
+    const int begin = int((int64_t(V) * r) / R), end = int((int64_t(V) * (r + 1)) / R);
+    int rc = rt_download(ctx[size_t(r)], RT_BUF_RGB8, spp, rgb.data() + image * size_t(begin), image * size_t(end - begin));
+    if (rc != RT_OK) die(ctx[size_t(r)], "rt_download", rc);
+  }
+  for (int v = 0; v < V; v++) {
+    std::printf("\rScanlines remaining: %d ", frame.image_height);
+    write_ppm_p3(*outs[size_t(v)], frame.image_width, frame.image_height, rgb.data() + image * size_t(v));
+    outs[size_t(v)]->flush();
+    std::printf("\rDone.                       \n");
+  }
+  std::fflush(stdout);
+}
+}  // namespace rtb200
 #endif  // RTB200_NO_RENDER_IMPL
 
 #endif  // RTB200_HOST_HPP

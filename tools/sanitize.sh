@@ -1,6 +1,6 @@
 #!/bin/bash
-# The library's own sanitizer run.  compute-sanitizer is CLOSED on this GPU pool ("runs under it have left GPUs needing a
-# reset" — the refusal is kept in profiles/sanitizer/compute_sanitizer_refused.txt), so the checks are compiled in:
+# The library's own sanitizer run.  compute-sanitizer is not available on the GPU machines (the refusal is kept in
+# profiles/sanitizer/compute_sanitizer_refused.txt), so the checks are compiled in:
 #   1. build/variants/checks.so = the library with -DRT_CHECKS=1: every dynamically indexed device access (BVH nodes,
 #      leaf references, primitive / material / texture / texel arrays, both traversal stacks, accumulator pixels) is
 #      bounds-checked on the device; a failure surfaces as RT_ERR_CUDA from the next rt_synchronize
@@ -13,7 +13,6 @@
 cd "$(dirname "$0")/.."
 OUT=gpurun_out/sanitizer
 mkdir -p $OUT
-compute-sanitizer --tool memcheck python -c "print(1)" > $OUT/compute_sanitizer_refused.txt 2>&1
 rc=0
 RT_B200_LIB=build/variants/checks.so RT_B200_DEBUG=1 python tools/sanitize_target.py > $OUT/checks_build.log 2>&1 || rc=1
 echo "checks build: rc=$rc, $(grep -c 'device-side checks evaluated' $OUT/checks_build.log) synchronisations reported, failures: $(grep -c 'worst failing site [1-9]' $OUT/checks_build.log)"

@@ -1,6 +1,7 @@
 """The workload compute-sanitizer runs over (tools/sanitize.sh): every kernel of the library on small inputs —
 smoke-sized parity queries, random-scene closest hits, 64-pixel renders of book2_final and cornell_smoke with every render
-kernel (and the instrumented variants), the push / adopt / peer paths with two contexts, finalize + downloads.
+kernel (and the instrumented variants), a batch of views (rt_render_views), the push / adopt / peer paths with two contexts,
+finalize + downloads.
 Asserts the kernels still agree with each other, so a sanitizer-induced timing change cannot hide a race."""
 import importlib, os, sys
 import numpy as np
@@ -55,9 +56,17 @@ for name, depth in (("book2_final", 40), ("cornell_smoke", 50), ("bouncing_spher
             print(name, tag, "refused:", e)
     for tag, a in acc.items():
         assert np.array_equal(a, acc["mega"]), (name, tag)
+    # a batch of views (render_kernel's VIEWS instantiation under this scene's plan): each view = its single render
+    views = [sc.camera_copy(image_width=WIDTH, samples_per_pixel=SPP, max_depth=md, vfov=30.0 + 5 * i) for i, md in enumerate((depth, 3, 0))]
+    ctx.render_views(views, seed=9)
+    batch = ctx.download_accum()
+    for i, v in enumerate(views):
+        ctx.render(v, seed=9)
+        assert np.array_equal(ctx.download_accum(), batch[i]), (name, "view", i)
     if os.environ.get("SAN_HASH"):
         import hashlib
         print("HASH", name, hashlib.sha1(acc["mega"].tobytes()).hexdigest()[:12], flush=True)
+        print("HASH", name, "views", hashlib.sha1(batch.tobytes()).hexdigest()[:12], flush=True)
     ctx.download_rgb8(SPP), ctx.download_radiance(SPP), ctx.stats()
     ctx.synchronize()  # a checks build reports failed device-side checks here
     print(name, "ok:", sorted(acc), flush=True)
