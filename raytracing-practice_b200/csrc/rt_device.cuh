@@ -13,6 +13,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include <type_traits>
 
 #include "device_scene.h"
 
@@ -337,7 +338,9 @@ __device__ __forceinline__ void load_node(const NodeSource& ns, int idx, float4&
 
 // Copies the first `n` BVH node records into shared memory.  With RT_NODE_CH and a fully staged BVH every (lo, hi) pair
 // becomes (centre, half extent) on the way, rounded so that [c - h, c + h] contains [lo, hi]: the box the traversal sees
-// never shrinks.
+// never shrinks.  The staged record is child-interleaved, {c0x c1x c0y c1y} {c0z c1z h0x h1x} {h0y h1y h0z h1z}
+// {child0 child1 - -}, so that each (child 0, child 1) pair of a value sits in two adjacent registers: the operand of
+// one packed FFMA2 in node_step.
 template <bool ALL_SMEM>
 __device__ __forceinline__ void stage_nodes(float4* s_nodes, const float4* __restrict__ g_nodes, int n) {
   if (RT_NODE_CH && ALL_SMEM) {
@@ -350,6 +353,8 @@ __device__ __forceinline__ void stage_nodes(float4* s_nodes, const float4* __res
       float4 a = g_nodes[4 * i], b = g_nodes[4 * i + 1], c = g_nodes[4 * i + 2];
       ch(a.x, a.w), ch(a.y, b.x), ch(a.z, b.y);  // child 0: x, y, z
       ch(b.z, c.y), ch(b.w, c.z), ch(c.x, c.w);  // child 1
+      const float4 q0 = make_float4(a.x, b.z, a.y, b.w), q1 = make_float4(a.z, c.x, a.w, c.y), q2 = make_float4(b.x, c.z, b.y, c.w);
+      a = q0, b = q1, c = q2;
       if (RT_NODE_PLANAR) {
         const float4 dd = g_nodes[4 * i + 3];
         s_nodes[i] = a, s_nodes[n + i] = b, s_nodes[2 * n + i] = c;
@@ -510,8 +515,7 @@ enum : int { CN_NODE = 0, CN_SPH = 1, CN_SPH_HIT = 2, CN_QUAD = 3, CN_QUAD_FULL 
 enum : int { MODE_SHADE = 0, MODE_NODE = 1, MODE_LEAF = 2, MODE_DONE = 3 };
 
 struct TravState {
-  float3 o, d, inv, ood;
-  float3 ainv;  // |1/d| (RT_NODE_CH node steps only; dead otherwise)
+  float3 o, d, inv, nood;  // nood = -o/d: the addend of the slab FFMA2 in node_step, which has no negation modifier
   float time, tmin;
   Hit best;
   uint32_t skip;  // the primitive the ray starts on (REF_NONE for camera rays / medium scatters)
@@ -604,8 +608,7 @@ __device__ __forceinline__ void trav_set_ray(TravState& ts, float3 o, float3 d, 
   ts.o = o, ts.d = d, ts.time = time, ts.tmin = tmin, ts.skip = skip;
   ts.inv = f3(fabsf(d.x) > 1e-30f ? rcp_fast(d.x) : copysignf(1e30f, d.x), fabsf(d.y) > 1e-30f ? rcp_fast(d.y) : copysignf(1e30f, d.y),
               fabsf(d.z) > 1e-30f ? rcp_fast(d.z) : copysignf(1e30f, d.z));
-  ts.ood = o * ts.inv;
-  ts.ainv = f3(fabsf(ts.inv.x), fabsf(ts.inv.y), fabsf(ts.inv.z));
+  ts.nood = -(o * ts.inv);
 }
 
 // The scene-enclosing media (met by every ray — the r=5000 fog of the Book-2 final scene) are not BVH leaves:
@@ -635,9 +638,9 @@ __device__ __forceinline__ Hit sample_global_media(const DeviceScene& sc, float3
 // boxes that are subsets of this one, and fma / min / max are monotone, so a miss here implies a miss at every
 // node: skipping the traversal for such rays cannot change any result.
 __device__ __forceinline__ bool ray_meets_scene(const DeviceScene& sc, const TravState& ts, float tmax) {
-  const float x0 = fmaf(sc.bounds_lo[0], ts.inv.x, -ts.ood.x), x1 = fmaf(sc.bounds_hi[0], ts.inv.x, -ts.ood.x);
-  const float y0 = fmaf(sc.bounds_lo[1], ts.inv.y, -ts.ood.y), y1 = fmaf(sc.bounds_hi[1], ts.inv.y, -ts.ood.y);
-  const float z0 = fmaf(sc.bounds_lo[2], ts.inv.z, -ts.ood.z), z1 = fmaf(sc.bounds_hi[2], ts.inv.z, -ts.ood.z);
+  const float x0 = fmaf(sc.bounds_lo[0], ts.inv.x, ts.nood.x), x1 = fmaf(sc.bounds_hi[0], ts.inv.x, ts.nood.x);
+  const float y0 = fmaf(sc.bounds_lo[1], ts.inv.y, ts.nood.y), y1 = fmaf(sc.bounds_hi[1], ts.inv.y, ts.nood.y);
+  const float z0 = fmaf(sc.bounds_lo[2], ts.inv.z, ts.nood.z), z1 = fmaf(sc.bounds_hi[2], ts.inv.z, ts.nood.z);
   const float n = fmaxf(fmaxf(fminf(x0, x1), fminf(y0, y1)), fmaxf(fminf(z0, z1), ts.tmin));
   const float f = fminf(fminf(fmaxf(x0, x1), fmaxf(y0, y1)), fminf(fmaxf(z0, z1), tmax));
   return n <= f;
@@ -661,32 +664,39 @@ __device__ __forceinline__ int node_step(TravState& ts, Stack& st, const NodeSou
   int c0, c1;
   load_node<ALL_SMEM>(ns, ts.cur, a, b, c, c0, c1);
   if (COUNT) cn[CN_NODE]++;
-  const float3 inv = ts.inv, ood = ts.ood;
+  const float3 inv = ts.inv, ood = -ts.nood;
   float n0, f0, n1, f1;
   if (RT_NODE_CH && ALL_SMEM) {
-    // Staged nodes hold (centre, half extent) per axis in the slots of (lo, hi) — see stage_nodes(): the slab's two
-    // plane distances are tc -+ h |1/d| with tc = (c - o)/d, so near and far need no per-axis min / max.  Three FFMA
-    // per axis and child instead of two FFMA + two FMNMX: the FMA and ALU pipes each take one warp instruction per two
-    // cycles (B300_MICROARCH.md, "fma vs alu split"), and the lo/hi form puts 28 of a node step's ~50 instructions on
-    // the ALU pipe against 12 on the FMA pipe; this form issues 6 fewer instructions and splits them 18 / 16.
-#if RT_NODE_CH == 2  // |1/d| through the operand modifier of FMUL: no extra registers, four FMA-pipe operations per axis
-    float tx = fmaf(a.x, inv.x, -ood.x), ty = fmaf(a.y, inv.y, -ood.y), tz = fmaf(a.z, inv.z, -ood.z);
-    float ex = a.w * fabsf(inv.x), ey = b.x * fabsf(inv.y), ez = b.y * fabsf(inv.z);
-    n0 = fmaxf(fmaxf(tx - ex, ty - ey), fmaxf(tz - ez, ts.tmin));
-    f0 = fminf(fminf(tx + ex, ty + ey), fminf(tz + ez, ts.best.t));
-    tx = fmaf(b.z, inv.x, -ood.x), ty = fmaf(b.w, inv.y, -ood.y), tz = fmaf(c.x, inv.z, -ood.z);
-    ex = c.y * fabsf(inv.x), ey = c.z * fabsf(inv.y), ez = c.w * fabsf(inv.z);
-    n1 = fmaxf(fmaxf(tx - ex, ty - ey), fmaxf(tz - ez, ts.tmin));
-    f1 = fminf(fminf(tx + ex, ty + ey), fminf(tz + ez, ts.best.t));
-#else
-    const float3 ai = ts.ainv;
-    float tx = fmaf(a.x, inv.x, -ood.x), ty = fmaf(a.y, inv.y, -ood.y), tz = fmaf(a.z, inv.z, -ood.z);
-    n0 = fmaxf(fmaxf(fmaf(-a.w, ai.x, tx), fmaf(-b.x, ai.y, ty)), fmaxf(fmaf(-b.y, ai.z, tz), ts.tmin));
-    f0 = fminf(fminf(fmaf(a.w, ai.x, tx), fmaf(b.x, ai.y, ty)), fminf(fmaf(b.y, ai.z, tz), ts.best.t));
-    tx = fmaf(b.z, inv.x, -ood.x), ty = fmaf(b.w, inv.y, -ood.y), tz = fmaf(c.x, inv.z, -ood.z);
-    n1 = fmaxf(fmaxf(fmaf(-c.y, ai.x, tx), fmaf(-c.z, ai.y, ty)), fmaxf(fmaf(-c.w, ai.z, tz), ts.tmin));
-    f1 = fminf(fminf(fmaf(c.y, ai.x, tx), fmaf(c.z, ai.y, ty)), fminf(fmaf(c.w, ai.z, tz), ts.best.t));
-#endif
+    // Staged nodes hold (centre, half extent) per axis, child-interleaved — see stage_nodes(): the slab's two plane
+    // distances are tc -+ h |1/d| with tc = (c - o)/d, so near and far need no per-axis min / max.  Each (child 0,
+    // child 1) pair of an axis is one packed FFMA2 with the per-lane 1/d, -o/d or |1/d| broadcast to both halves; per
+    // component it is the scalar FFMA(.FTZ) of the unpaired form, same operands, same rounding, so the bits are those of
+    // three scalar FFMA per axis and child.  FFMA2 has no negation modifier, so packed near planes need -|1/d| in three
+    // registers of their own.  That pays in the local-stack plan (the large BVHs: +5 % on C5) and loses 3-5 % in the
+    // shared-memory-stack plan of the small scenes (C3a, C3b), which already spills more: there the near planes stay
+    // scalar FFMA with the -|.| operand modifier (profiles/r5_ffma2.md).
+    constexpr bool kPackNear = !std::is_same<Stack, TravStackS>::value;
+    const float2 tx = __ffma2_rn(make_float2(a.x, a.y), make_float2(inv.x, inv.x), make_float2(ts.nood.x, ts.nood.x));
+    const float2 ty = __ffma2_rn(make_float2(a.z, a.w), make_float2(inv.y, inv.y), make_float2(ts.nood.y, ts.nood.y));
+    const float2 tz = __ffma2_rn(make_float2(b.x, b.y), make_float2(inv.z, inv.z), make_float2(ts.nood.z, ts.nood.z));
+    const float2 hx = make_float2(b.z, b.w), hy = make_float2(c.x, c.y), hz = make_float2(c.z, c.w);
+    const float3 ai = f3(fabsf(inv.x), fabsf(inv.y), fabsf(inv.z));
+    const float2 fx = __ffma2_rn(hx, make_float2(ai.x, ai.x), tx), fy = __ffma2_rn(hy, make_float2(ai.y, ai.y), ty),
+                 fz = __ffma2_rn(hz, make_float2(ai.z, ai.z), tz);
+    float2 nx, ny, nz;
+    if constexpr (kPackNear) {
+      const float3 nai = f3(-fabsf(inv.x), -fabsf(inv.y), -fabsf(inv.z));
+      nx = __ffma2_rn(hx, make_float2(nai.x, nai.x), tx), ny = __ffma2_rn(hy, make_float2(nai.y, nai.y), ty);
+      nz = __ffma2_rn(hz, make_float2(nai.z, nai.z), tz);
+    } else {
+      nx = make_float2(fmaf(hx.x, -fabsf(inv.x), tx.x), fmaf(hx.y, -fabsf(inv.x), tx.y));
+      ny = make_float2(fmaf(hy.x, -fabsf(inv.y), ty.x), fmaf(hy.y, -fabsf(inv.y), ty.y));
+      nz = make_float2(fmaf(hz.x, -fabsf(inv.z), tz.x), fmaf(hz.y, -fabsf(inv.z), tz.y));
+    }
+    n0 = fmaxf(fmaxf(nx.x, ny.x), fmaxf(nz.x, ts.tmin));
+    f0 = fminf(fminf(fx.x, fy.x), fminf(fz.x, ts.best.t));
+    n1 = fmaxf(fmaxf(nx.y, ny.y), fmaxf(nz.y, ts.tmin));
+    f1 = fminf(fminf(fx.y, fy.y), fminf(fz.y, ts.best.t));
   } else {
     // slab test of both children (aabb.hpp:61-112), conservative: keep when tnear <= tfar
     float x0 = fmaf(a.x, inv.x, -ood.x), x1 = fmaf(a.w, inv.x, -ood.x);
@@ -724,7 +734,7 @@ __device__ __forceinline__ void node_step_spec(TravState& ts, TravStack& st, con
   int c0, c1;
   load_node<ALL_SMEM>(ns, ts.cur, a, b, c, c0, c1);
   if (COUNT) cn[CN_NODE]++;
-  const float3 inv = ts.inv, ood = ts.ood;
+  const float3 inv = ts.inv, ood = -ts.nood;
   float x0 = fmaf(a.x, inv.x, -ood.x), x1 = fmaf(a.w, inv.x, -ood.x);
   float y0 = fmaf(a.y, inv.y, -ood.y), y1 = fmaf(b.x, inv.y, -ood.y);
   float z0 = fmaf(a.z, inv.z, -ood.z), z1 = fmaf(b.y, inv.z, -ood.z);
@@ -796,7 +806,7 @@ __device__ __forceinline__ void leaf_body(TravState& ts, int leaf, const DeviceS
         const float4 b0 = STAGED ? lds_f4(ls.boxes + 48u * b) : __ldg(sc.boxes + 3 * b);
         const float4 b1 = STAGED ? lds_f4(ls.boxes + 48u * b + 16u) : __ldg(sc.boxes + 3 * b + 1);
         const float4 b2 = STAGED ? lds_f4(ls.boxes + 48u * b + 32u) : __ldg(sc.boxes + 3 * b + 2);
-        t = hit_box(b0, b1, b2, o, d, ts.inv, ts.ood, ts.tmin, ts.best.t, self_face, face);
+        t = hit_box(b0, b1, b2, o, d, ts.inv, -ts.nood, ts.tmin, ts.best.t, self_face, face);
         if (COUNT) cn[CN_BOX]++;
         ref = make_ref(REF_BOX, (b << 3) | uint32_t(face));
       }

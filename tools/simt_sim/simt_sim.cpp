@@ -35,6 +35,7 @@
 #include "../../raytracing-practice_b200/csrc/device_scene.h"
 inline float4 make_float4(float x, float y, float z, float w) { return float4{x, y, z, w}; }
 inline float2 make_float2(float x, float y) { return float2{x, y}; }
+inline float2 __ffma2_rn(float2 a, float2 b, float2 c) { return float2{std::fma(a.x, b.x, c.x), std::fma(a.y, b.y, c.y)}; }
 #include "../../raytracing-practice_b200/csrc/rt_device.cuh"
 #include "../../raytracing-practice_b200/csrc/scene_build.hpp"
 
@@ -295,7 +296,7 @@ static int sim_leaf_step(Job& J, std::vector<Engine*>& lanes, std::vector<Path*>
           const uint32_t b = idx >> 3;
           const int self_face = ((p.skip >> 30) == REF_BOX && p.skip != REF_NONE && ((p.skip & 0x3FFFFFFFu) >> 3) == b) ? int(p.skip & 7u) : -1;
           int face = 0;
-          t = hit_box(sc.boxes[3 * b], sc.boxes[3 * b + 1], sc.boxes[3 * b + 2], ts.o, ts.d, ts.inv, ts.ood, ts.tmin, ts.best.t, self_face, face);
+          t = hit_box(sc.boxes[3 * b], sc.boxes[3 * b + 1], sc.boxes[3 * b + 2], ts.o, ts.d, ts.inv, -ts.nood, ts.tmin, ts.best.t, self_face, face);
           ref = make_ref(REF_BOX, (b << 3) | uint32_t(face));
           c_box++;
         }
